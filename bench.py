@@ -2,6 +2,7 @@
 """Benchmark of the embedding -> interaction -> sparse-update hot path on B200 (contract: the task brief, section 4).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c2|c1|c3|c4|c5|rank] [--impl reference] [--dist uniform|zipf]
+                    [--dump-outputs DIR]
 
 Default workload = BASELINE.json configs[1] ("C2", the config the metric is quoted on): FM second-order + FFM on synthetic
 Criteo-shaped data -- 26 sparse fields, D = 16, batch 65536 per GPU, the public Criteo-Kaggle cardinalities (33.76 M rows;
@@ -291,10 +292,11 @@ def run_reference(args):
 
 
 # ====================================================================================================== GPU legs
-def run_legs(step, pool, B, args, world, dev, local, graph_step=None, extra_warmup=0, e2e_steps=None):
+def run_legs(step, pool, B, args, world, dev, local, graph_step=None, extra_warmup=0, e2e_steps=None, after_timed=None):
     """Device-resident leg (eager, per-kernel CUDA events, launch count) + end-to-end leg (inputs from pinned host memory on a
     copy stream, loss copied back every step; `graph_step` replays the same step as a CUDA graph when given).
-    step(inputs tuple, y) -> loss tensor.  Returns a dict of raw measurements (times already max-reduced over ranks)."""
+    step(inputs tuple, y) -> loss tensor.  `after_timed()` runs once right after the timed steps, before any further step
+    changes the models.  Returns a dict of raw measurements (times already max-reduced over ranks)."""
     import torch.distributed as dist
     from deeplearningrecommendationsystem_b200 import ops
 
@@ -319,6 +321,8 @@ def run_legs(step, pool, B, args, world, dev, local, graph_step=None, extra_warm
     ms_total = e0.elapsed_time(e1)
     gpu_launches = ops.launches() - launches0
     last_loss_eager = float(loss.detach())
+    if after_timed is not None:
+        after_timed()
     # per-kernel CUDA-event times come from a few EXTRA steps outside the timed region: bracketing every C-ABI call with two
     # events costs host time that the timed steps should not pay
     n_prof = min(args.steps, 5)
@@ -466,16 +470,27 @@ def build_c2(cards, dev, world, exchange=None, fabric=None):
     return fm, ffm, trainers, loss_fn
 
 
-def c2_job(cards, B, dist_name, dev, world, rank, args, local, n_pool=8, graph=True):
-    """-> (legs, n_uniq of one batch, models) for the FM + FFM step on `cards`"""
+DUMP_ROWS = 8192      # table rows sampled by --dump-outputs: 8192 x 416 floats of FFM = 13.6 MB
+
+
+def c2_job(cards, B, dist_name, dev, world, rank, args, local, n_pool=8, graph=True, dump_dir=None):
+    """-> (legs, n_uniq of one batch) for the FM + FFM step on `cards`.  With `dump_dir`, the outputs of the last
+    timed step are written there as .npy files (see dump_c2_outputs)."""
     from deeplearningrecommendationsystem_b200 import ops
     fm, ffm, trainers, loss_fn = build_c2(cards, dev, world)
+    if dump_dir is not None and fm.sharded:
+        raise ValueError("--dump-outputs samples rows of unsharded tables: run it on one GPU")
     pool = [((i,), y) for i, y in (make_ids(cards, B, 1234 + rank * 100 + k, dist_name, dev) for k in range(n_pool))]
 
     def step(ins, y):
         for tr in trainers:
             tr.train_loop(ins[0], train_rating=y)
         return trainers[0].train_loss
+
+    after_timed = None
+    if dump_dir is not None:
+        def after_timed():
+            dump_c2_outputs(dump_dir, trainers, (ffm, fm), pool[(args.steps - 1) % len(pool)][0][0])
 
     gstep = None
     if graph and (world == 1 or os.environ.get("RS_GRAPH_SHARDED", "1") == "1"):
@@ -486,12 +501,34 @@ def c2_job(cards, B, dist_name, dev, world, rank, args, local, n_pool=8, graph=T
             for tr in trainers:   # drop the eager leg's autograd graphs: their AccumulateGrad nodes are bound to its stream
                 tr.predictions_train = tr.train_loss = None
             return gs(ins[0], rating=y)[1]
-    legs = run_legs(step, pool, B, args, world, dev, local, graph_step=gstep, extra_warmup=3 if world > 1 else 0)
+    legs = run_legs(step, pool, B, args, world, dev, local, graph_step=gstep, extra_warmup=3 if world > 1 else 0,
+                    after_timed=after_timed)
     segs = ops.dedup_sort(pool[0][0][0], F, fm.offsets_host, fm.total_rows)
     n_uniq = segs.n_uniq
     del trainers, fm, ffm, pool
     torch.cuda.empty_cache()
     return legs, n_uniq
+
+
+def dump_c2_outputs(out_dir, trainers, models, ids):
+    """Write what the caller of the timed FFM + FM step holds after its last step, as float32 .npy files: each model's
+    predictions (B x 1), loss and bias, and the rows of its table at DUMP_ROWS lookups of the last batch `ids` (the rows
+    that step updated), picked by a fixed seed.  The inputs and the initial tables are seeded, so two builds run with the
+    same arguments can be compared file by file."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    n = ids.numel()
+    pick = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:DUMP_ROWS]
+    offsets = torch.tensor(models[0].offsets_host, dtype=torch.int64)
+    rows = (ids.reshape(-1)[pick.to(ids.device)].cpu() + offsets[pick % ids.shape[1]]).to(ids.device)
+    out = {}
+    for name, tr, m in zip(("ffm", "fm"), trainers, models):
+        out[f"{name}_predictions"] = tr.predictions_train
+        out[f"{name}_loss"] = tr.train_loss.reshape(1)
+        out[f"{name}_bias"] = m.bias
+        out[f"{name}_table_rows"] = m.weight[rows]
+    for name, t in out.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.detach().float().cpu().numpy())
 
 
 def c2_rooflines(legs, B, n_uniq, tag):
@@ -598,7 +635,7 @@ def run_c2(args):
     B = args.batch
     graph = args.graph
     progress(f"c2 headline: tables built, world={world}")
-    legs, n_uniq = c2_job(cards, B, args.dist, dev, world, rank, args, local, graph=graph)
+    legs, n_uniq = c2_job(cards, B, args.dist, dev, world, rank, args, local, graph=graph, dump_dir=args.dump_outputs)
     progress(f"c2 headline done: {legs['ms_step']:.3f} ms eager, {legs['ms_e2e']:.3f} ms e2e")
     line = base_line(args, world, B, legs, WORKLOADS["c2"],
                      {"fields": F, "dim": D, "rows": sum(cards), "ids": args.dist, "light": bool(args.light),
@@ -945,7 +982,12 @@ def main():
     ap.add_argument("--no-graph", dest="graph", action="store_false", help="eager Trainer.train_loop in the end-to-end leg too")
     ap.add_argument("--workload", default="c2", choices=["c2", "c1", "c3", "c4", "c5", "rank"],
                     help="c2 = headline (BASELINE.json configs[1]); c1/c3/c4/c5 = the other configs, one line per model")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="c2, one GPU: write the outputs of the last timed step (predictions, losses, biases, a fixed sample of "
+                         "updated table rows) to DIR/<name>.npy as float32")
     args = ap.parse_args()
+    if args.dump_outputs is not None and (args.impl != "b200" or args.workload != "c2"):
+        ap.error("--dump-outputs covers the c2 workload of the GPU implementation")
     if args.impl == "reference":
         if args.workload == "rank":
             args.workload = "c2"
