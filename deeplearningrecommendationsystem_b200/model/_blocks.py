@@ -106,9 +106,20 @@ class RowSink:
         self.pending.append((grp, [w._rs_field for w in weights], ids, dE))
 
     def apply(self, opt):
-        for grp, fields, ids, dE in self.pending:
-            F, W = len(fields), grp["buf"].shape[1]
-            offs = [grp["offsets"][f] for f in fields]
+        entries = self.pending
+        if opt.kind != "sgd" or opt.weight_decay != 0.0:
+            # Adam's moments and the decay term advance once per step: the lookups of several forwards into one group are
+            # merged into one update over global rows (F = 1) on the summed gradient
+            by_grp = {}
+            for e in entries:
+                by_grp.setdefault(id(e[0]), []).append(e)
+            entries = [es[0] if len(es) == 1 else self._merged(es) for es in by_grp.values()]
+        for grp, fields, ids, dE in entries:
+            W = grp["buf"].shape[1]
+            if fields is None:                  # merged entry: ids are global rows of the group's buffer
+                F, offs = 1, None
+            else:
+                F, offs = len(fields), [grp["offsets"][f] for f in fields]
             segs = ops.dedup_sort(ids.reshape(-1, F), F, offs, sum(grp["rows"]), max_width=W)
             if opt.kind == "sgd":
                 ops.segment_update(segs, ops.RS_UPD_SGD, W, F, dense=dE.reshape(-1, W), table=grp["buf"], lr=opt.lr, wd=opt.weight_decay)
@@ -118,6 +129,16 @@ class RowSink:
                 ops.segment_update(segs, ops.RS_UPD_ADAM, W, F, dense=dE.reshape(-1, W), table=grp["buf"], m=grp["m"], v=grp["v"],
                                    lr=opt.lr, wd=opt.weight_decay, betas=opt.betas, eps=opt.eps, step=opt.step_count)
         self.pending.clear()
+
+    @staticmethod
+    def _merged(entries):
+        grp, W = entries[0][0], entries[0][0]["buf"].shape[1]
+        keys, rows = [], []
+        for _, fields, ids, dE in entries:
+            offs = torch.tensor([grp["offsets"][f] for f in fields], dtype=torch.int64, device=ids.device)
+            keys.append((ids.reshape(-1, len(fields)) + offs).reshape(-1))
+            rows.append(dE.reshape(-1, W))
+        return grp, None, torch.cat(keys), torch.cat(rows)
 
 
 class FusedRows:

@@ -259,10 +259,30 @@ class _FieldModel(nn.Module):
             ops.segment_update(segs, ops.RS_UPD_ADAM, self.width, F, table=self.weight.data, m=self.adam_m, v=self.adam_v,
                                lr=opt.lr, wd=opt.weight_decay, betas=opt.betas, eps=opt.eps, step=opt.step_count, tag=tag, **src)
 
+    def _merged_record(self, recs):
+        """The pending records of several forwards as one record over their concatenated batches, so that Adam and weight
+        decay step once on the summed gradient (see FusedRowOptimizer).  Stash + per-sample scale are concatenated as they
+        are when every record has them; otherwise the stashed rows are multiplied out into per-lookup gradient rows (the
+        same fp32 product the update kernels form)."""
+        ids = torch.cat([r["ids"] for r in recs])
+        if all(r.get("stash") is not None for r in recs):
+            return {"ids": ids, "stash": torch.cat([r["stash"] for r in recs]), "g": torch.cat([r["g"] for r in recs])}
+        dense = [r["g"].reshape(r["ids"].shape[0], -1, self.width) if r.get("stash") is None else
+                 r["stash"].reshape(r["ids"].shape[0], -1, self.width) * r["g"].reshape(-1, 1, 1) for r in recs]
+        return {"ids": ids, "stash": None, "g": torch.cat(dense)}
+
     def apply_pending(self, opt):
-        for rec in self._pending.values():
-            if "g" not in rec:
-                continue
+        recs = [rec for rec in self._pending.values() if "g" in rec]
+        if len(recs) > 1 and (opt.kind != "sgd" or opt.weight_decay != 0.0):
+            # several forwards before one step: Adam's moments and the decay term must advance once, on the summed gradient
+            if self.sharded:
+                raise RuntimeError("a row-sharded table takes one forward per optimizer step with Adam or weight_decay != 0 "
+                                   f"({len(recs)} forwards are pending)")
+            if any(r.get("recompute") for r in recs):
+                raise RuntimeError("a forward without a Jacobian stash cannot be merged with another one before a step with "
+                                   "weight_decay != 0; run with RS_FFM_RECOMPUTE=0")
+            recs = [self._merged_record(recs)]
+        for rec in recs:
             src = {"dense": rec["g"]} if rec.get("stash") is None else {"stash": rec["stash"], "scale": rec["g"]}
             if not self.sharded:
                 segs = ops.dedup_sort(rec["ids"], self.F, self.offsets_host, self.total_rows, max_width=self.width)

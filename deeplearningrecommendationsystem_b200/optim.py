@@ -16,6 +16,13 @@ from . import ops
 
 
 class FusedRowOptimizer:
+    """One ``step()`` is one optimizer step per table, also when the model ran several forwards since ``zero_grad()``.
+    With ``kind="adam"`` or ``weight_decay != 0`` the pending lookups of a table are merged and updated once on their
+    summed gradient, as ``torch.optim`` steps once on the accumulated ``.grad``: the moments advance once and the decay
+    term is applied once.  Plain SGD without decay applies the forwards one after another (the same result up to
+    rounding).  A row-sharded table takes one forward per step with Adam or weight decay (several raise), and so does
+    the stash-free FFM forward (``RS_FFM_RECOMPUTE=1``) with weight decay."""
+
     def __init__(self, model, dense_optimizer=None, lr=0.01, kind="sgd", weight_decay=0.0, betas=(0.9, 0.999), eps=1e-8,
                  data_parallel=True):
         """data_parallel: average the dense parameters' gradients over the process group before the dense step (the

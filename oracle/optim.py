@@ -40,9 +40,12 @@ def sgd_rows(table, ids, G, lr):
     return table
 
 
-def adam_rows(table, m, v, ids, G, step, lr=1e-3, b1=0.9, b2=0.999, eps=1e-8):
-    """Lazy (row-sparse) Adam: only touched rows update their moments and weights."""
+def adam_rows(table, m, v, ids, G, step, lr=1e-3, b1=0.9, b2=0.999, eps=1e-8, wd=0.0):
+    """Lazy (row-sparse) Adam: only touched rows update their moments and weights.  wd: L2 decay folded into the
+    summed gradient of each touched row, as torch.optim.Adam(weight_decay=wd) does."""
     uniq, g = segment_sum_rows(ids, G)
+    if wd != 0.0:
+        g = g.add(table[uniq], alpha=wd)
     mu = torch.lerp(m[uniq], g, 1.0 - b1)
     vu = b2 * v[uniq] + (1.0 - b2) * g * g
     bc1 = 1.0 - b1 ** step
