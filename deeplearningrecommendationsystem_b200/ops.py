@@ -752,11 +752,16 @@ def afm_bwd(E, W, b, h, attw, g_pooled, impl="auto", return_masks=False):
         n = parts.value
         Up = torch.empty(n, D, A, dtype=torch.float32, device=E.device)
         m1p = torch.empty(n, A, dtype=torch.float32, device=E.device)
-        # the workspace (ds, mask bits, dP: 3.1 GB at C3) is cached per device instead of being allocated every backward
-        ws = _afm_ws.get(E.device)
-        if ws is None or ws.numel() < nbytes.value:
-            _afm_ws[E.device] = None
-            ws = _afm_ws[E.device] = torch.empty(nbytes.value, dtype=torch.uint8, device=E.device)
+        # the workspace (ds, mask bits, dP: 3.1 GB at C3) is cached per device instead of being allocated every backward.
+        # A CUDA-graph capture gets a workspace of its own from the graph's private pool: a cached block is dropped when a
+        # larger shape arrives and handed to other tensors, which the replays would then overwrite.
+        if torch.cuda.is_current_stream_capturing():
+            ws = torch.empty(nbytes.value, dtype=torch.uint8, device=E.device)
+        else:
+            ws = _afm_ws.get(E.device)
+            if ws is None or ws.numel() < nbytes.value:
+                _afm_ws[E.device] = None
+                ws = _afm_ws[E.device] = torch.empty(nbytes.value, dtype=torch.uint8, device=E.device)
         with _timed("afm_bwd_tc"):
             _lib.check(lib.rs_afm_bwd_tc(E.data_ptr(), B, F, D, A, W.data_ptr(), b.data_ptr(), h.data_ptr(), attw.data_ptr(),
                                          g_pooled.data_ptr(), dE.data_ptr(), Up.data_ptr(), m1p.data_ptr(), n, ws.data_ptr(),

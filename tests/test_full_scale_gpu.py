@@ -143,16 +143,16 @@ def zipf_ids(c, shape, g, device, a=1.05):
     return (x.floor().long() - 1).clamp_(0, c - 1)
 
 
-def make_batch(cards, dist, seed):
-    """(B, F) local ids drawn as bench.py draws them, with samples pinned to row 0 and to row card - 1 of every field
+def make_batch(cards, dist, seed, nb=B):
+    """(nb, F) local ids drawn as bench.py draws them, with samples pinned to row 0 and to row card - 1 of every field
     (the last row of the last field is the highest address in the table), and Bernoulli(0.3) labels."""
     g = torch.Generator(device="cuda").manual_seed(seed)
-    cols = [zipf_ids(c, (B,), g, "cuda") if dist == "zipf" else torch.randint(0, c, (B,), generator=g, device="cuda") for c in cards]
+    cols = [zipf_ids(c, (nb,), g, "cuda") if dist == "zipf" else torch.randint(0, c, (nb,), generator=g, device="cuda") for c in cards]
     ids = torch.stack(cols, dim=1).contiguous()
     last = torch.tensor(cards, device="cuda") - 1
-    ids[0], ids[B // 2] = 0, 0
-    ids[1], ids[B - 1], ids[B // 3] = last, last, last
-    y = (torch.rand(B, generator=g, device="cuda") < 0.3).float()
+    ids[0], ids[nb // 2] = 0, 0
+    ids[1], ids[nb - 1], ids[nb // 3] = last, last, last
+    y = (torch.rand(nb, generator=g, device="cuda") < 0.3).float()
     return ids, y
 
 
