@@ -118,6 +118,8 @@ SIGNATURES = {
     "rs_ffm_fwd_train": [_PP(rs_tables), _P, _L, _I, C.c_uint64, _P, _P, _P, _P],
     "rs_ffm_bwd_update": [_PP(rs_tables), _P, _L, _I, C.c_uint64, _P, _PP(rs_segments), _PP(rs_update), _P, _Z, _P, _P],
     "rs_replica_sgd": [_PP(_P), _PP(_P), _L, _I, _I, _F, _F, _P],
+    "rs_mark_rows": [_PP(rs_segments), _L, _P, _L, _P, _P],
+    "rs_replica_update": [_PP(_P), _PP(_P), _PP(_P), _L, _I, _I, _PP(rs_update), _P],
     "rs_adam_dense": [_P, _P, _P, _P, _L, _F, _F, _F, _F, _F, _I, _P],
     "rs_xembed_fwd": [_PP(rs_xslots), _P, _L, _P, _P, _P],
     "rs_xembed_bag_bwd": [_PP(rs_xslots), _P, _P, _L, _PP(_P), _P, _Z, _P],

@@ -621,6 +621,18 @@ int launch_mode(const UpdParams &P, int mode, int64_t n, cudaStream_t st) {
 
 namespace rs {
 
+void set_opt_scalars(const rs_update *u, UpdParams &P) {
+  P.lr = u->lr;
+  P.wd = u->wd;
+  P.beta1 = u->beta1;
+  P.beta2 = u->beta2;
+  P.eps = u->eps;
+  double bc1 = 1.0 - pow((double)u->beta1, (double)u->step);
+  double bc2 = 1.0 - pow((double)u->beta2, (double)u->step);
+  P.step_size = (float)((double)u->lr / (bc1 > 0 ? bc1 : 1.0));
+  P.inv_sqrt_bc2 = (float)(1.0 / sqrt(bc2 > 0 ? bc2 : 1.0));
+}
+
 int make_upd_params(const rs_segments *seg, int64_t n, const rs_update *u, UpdParams &P) {
   RS_CHECK_ARG((int64_t)(2 * (n / RS_CHUNK + 2)) * u->width <= seg->partial_floats, RS_E_WORKSPACE,
                "rs_segment_update: dedup workspace was sized for a narrower row (need %lld floats of partials, have %lld)",
@@ -658,15 +670,7 @@ int make_upd_params(const rs_segments *seg, int64_t n, const rs_update *u, UpdPa
   P.W = u->width;
   P.F = u->F;
   P.scale_width = u->scale_width;
-  P.lr = u->lr;
-  P.wd = u->wd;
-  P.beta1 = u->beta1;
-  P.beta2 = u->beta2;
-  P.eps = u->eps;
-  double bc1 = 1.0 - pow((double)u->beta1, (double)u->step);
-  double bc2 = 1.0 - pow((double)u->beta2, (double)u->step);
-  P.step_size = (float)((double)u->lr / (bc1 > 0 ? bc1 : 1.0));
-  P.inv_sqrt_bc2 = (float)(1.0 / sqrt(bc2 > 0 ? bc2 : 1.0));
+  set_opt_scalars(u, P);
   P.use_stream = 0;
   P.combine_only = 0;
   P.half_sm = u->half_sm;

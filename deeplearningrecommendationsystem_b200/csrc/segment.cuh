@@ -25,13 +25,15 @@ __device__ __forceinline__ float upd_sgd(float w, float g, const UpdParams &P) {
 __device__ __forceinline__ float4 upd_sgd(float4 w, float4 g, const UpdParams &P) {
   return make_float4(upd_sgd(w.x, g.x, P), upd_sgd(w.y, g.y, P), upd_sgd(w.z, g.z, P), upd_sgd(w.w, g.w, P));
 }
-// torch.optim.Adam single-tensor arithmetic on one element
+// torch.optim.Adam single-tensor arithmetic on one element.  Every rounding is spelled out (the FMA contraction nvcc
+// chose for the row-update kernels): left to the compiler, the same source contracts differently in different kernels
+// (v = fma(g, (1-b2) g, b2 v) instead of fma(b2, v, ((1-b2) g) g)), and every kernel that calls this must give the same bits.
 __device__ __forceinline__ void adam1(float &w, float &m, float &v, float g, const UpdParams &P) {
-  g = g + P.wd * w;
-  m = m + (1.0f - P.beta1) * (g - m);  // lerp_(g, 1-beta1)
-  v = P.beta2 * v + (1.0f - P.beta2) * g * g;
-  float denom = sqrtf(v) * P.inv_sqrt_bc2 + P.eps;
-  w = w - P.step_size * (m / denom);
+  g = __fmaf_rn(P.wd, w, g);                                          // g + wd*w
+  m = __fmaf_rn(1.0f - P.beta1, __fsub_rn(g, m), m);                  // lerp_(g, 1-beta1)
+  v = __fmaf_rn(P.beta2, v, __fmul_rn(__fmul_rn(1.0f - P.beta2, g), g));
+  const float denom = __fmaf_rn(sqrtf(v), P.inv_sqrt_bc2, P.eps);     // sqrt(v) / sqrt(bc2) + eps
+  w = __fmaf_rn(-__fdiv_rn(m, denom), P.step_size, w);                // w - step_size * m / denom
 }
 
 // Slot of a chunk's partial sum.  Full chunks are disjoint runs of RS_CHUNK sorted lookups, so start/RS_CHUNK is
@@ -39,6 +41,9 @@ __device__ __forceinline__ void adam1(float &w, float &m, float &v, float g, con
 // start/RS_CHUNK is unique among tails as well.  Even slots hold full chunks, odd slots tails.
 __device__ __forceinline__ int partial_slot(int start, int len) { return 2 * (start / RS_CHUNK) + (len < RS_CHUNK ? 1 : 0); }
 
+// Adam's bias-correction scalars of step u->step (and lr, wd, betas, eps) into P: the one host computation behind every
+// lazy row update (rs_segment_update, rs_replica_update), so their arithmetic cannot drift apart.
+void set_opt_scalars(const rs_update *u, UpdParams &P);
 int fill_routes(Routes &R, const rs_routes *r, const char *who);
 int launch_seg_stream(const UpdParams &P, int64_t n, int mode, cudaStream_t st);
 int make_upd_params(const rs_segments *seg, int64_t n, const rs_update *u, UpdParams &P);   // segment.cu

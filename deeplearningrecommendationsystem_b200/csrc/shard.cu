@@ -14,7 +14,7 @@
 #include <stdlib.h>
 #include <string.h>
 
-#include "common.cuh"
+#include "segment.cuh"
 
 namespace {
 
@@ -291,6 +291,82 @@ __global__ void __launch_bounds__(256) replica_sgd_kernel(const __grid_constant_
   }
 }
 
+// ------------------------------------------------------------------ replicated small tables: lazy row update (SGD / Adam)
+// Same slicing, rank-ordered sum and store into every replica as replica_sgd_kernel, but only rows that some rank's batch
+// touched move (touched[r][row] != 0 for some r) -- the single-GPU row update is lazy, and an untouched row must keep its
+// bits under Adam (m != 0 keeps moving w) and weight decay.  The flags decide, not the gradient: a touched row whose summed
+// gradient is exactly zero still steps.  The arithmetic is the row-update kernels' (upd_sgd / adam1, segment.cuh).
+// Adam's m and v are not replicated: only this rank's slice exists, indexed from lo4.
+struct Flags {
+  const uint8_t *t[RS_MAX_RANKS];
+};
+
+template <int MODE>
+__global__ void __launch_bounds__(256) replica_update_kernel(const __grid_constant__ Replicas R, const __grid_constant__ Flags T, int world,
+                                                            int rank, int64_t lo4, int64_t hi4, int wv, float *__restrict__ m_slice,
+                                                            float *__restrict__ v_slice, float lr, float wd, float beta1, float beta2,
+                                                            float eps, float step_size, float inv_sqrt_bc2) {
+  rs::UpdParams P;
+  P.lr = lr;
+  P.wd = wd;
+  P.beta1 = beta1;
+  P.beta2 = beta2;
+  P.eps = eps;
+  P.step_size = step_size;
+  P.inv_sqrt_bc2 = inv_sqrt_bc2;
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+  for (int64_t i = lo4 + (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < hi4; i += stride) {
+    // width % 4 == 0: a float4 never straddles two rows (32-bit division where it fits: the 64-bit one is emulated)
+    const int64_t row = hi4 <= 0xffffffffll ? (int64_t)((uint32_t)i / (uint32_t)wv) : i / wv;
+    uint32_t hit = 0;
+    for (int r0 = 0; r0 < world; r0 += 8) {
+      uint32_t f[8];
+#pragma unroll
+      for (int k = 0; k < 8; ++k) f[k] = (r0 + k < world) ? T.t[r0 + k][row] : 0u;
+#pragma unroll
+      for (int k = 0; k < 8; ++k) hit |= f[k];
+    }
+    if (!hit) continue;
+    float4 acc = rs::f4_zero();
+    for (int r0 = 0; r0 < world; r0 += 8) {      // replica_sgd_kernel's sum: eight peer loads in flight, rank order
+      float4 v[8];
+#pragma unroll
+      for (int k = 0; k < 8; ++k) v[k] = (r0 + k < world) ? rs::ldg_f4(R.g[r0 + k] + i * 4) : rs::f4_zero();
+#pragma unroll
+      for (int k = 0; k < 8; ++k)
+        if (r0 + k < world) acc = rs::f4_add(acc, v[k]);
+    }
+    float4 w = rs::ldg_f4(R.w[rank] + i * 4);
+    if (MODE == RS_UPD_SGD) {
+      w = rs::upd_sgd(w, acc, P);
+    } else {
+      float *mp = m_slice + (i - lo4) * 4, *vp = v_slice + (i - lo4) * 4;
+      float4 m = rs::ldg_f4(mp), v = rs::ldg_f4(vp);
+      rs::adam1(w.x, m.x, v.x, acc.x, P);
+      rs::adam1(w.y, m.y, v.y, acc.y, P);
+      rs::adam1(w.z, m.z, v.z, acc.z, P);
+      rs::adam1(w.w, m.w, v.w, acc.w, P);
+      rs::stg_f4(mp, m);
+      rs::stg_f4(vp, v);
+    }
+    for (int r = 0; r < world; ++r) rs::stg_f4(R.w[(rank + r) % world] + i * 4, w);
+  }
+}
+
+__global__ void __launch_bounds__(256) mark_rows_kernel(const int64_t *__restrict__ uniq, const int32_t *__restrict__ n_uniq,
+                                                       uint8_t *__restrict__ touched, int64_t rows, int32_t *status) {
+  const int64_t nu = *n_uniq;
+  for (int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; j < nu; j += (int64_t)gridDim.x * blockDim.x)
+    touched[rs::clamp_id(uniq[j], rows, status)] = 1;
+}
+
+// rank `rank`'s float4 slice [lo4, hi4) of n4: per = ceil(n4 / world)
+void replica_slice(int64_t n4, int world, int rank, int64_t &lo4, int64_t &hi4) {
+  const int64_t per = (n4 + world - 1) / world;
+  lo4 = per * rank < n4 ? per * rank : n4;
+  hi4 = lo4 + per < n4 ? lo4 + per : n4;
+}
+
 }  // namespace
 
 RS_API int rs_replica_sgd(float *const *w, const float *const *g, int64_t numel, int32_t world, int32_t rank, float lr, float wd,
@@ -303,12 +379,58 @@ RS_API int rs_replica_sgd(float *const *w, const float *const *g, int64_t numel,
     R.w[k] = w[k];
     R.g[k] = g[k];
   }
-  const int64_t n4 = numel / 4, per = (n4 + world - 1) / world;
-  const int64_t lo4 = per * rank < n4 ? per * rank : n4, hi4 = lo4 + per < n4 ? lo4 + per : n4;
+  int64_t lo4, hi4;
+  replica_slice(numel / 4, world, rank, lo4, hi4);
   if (hi4 <= lo4) return RS_OK;
   int64_t blocks = (hi4 - lo4 + 255) / 256;
   const int cap = rs::num_sms() * 8;
   replica_sgd_kernel<<<(int)(blocks < cap ? blocks : cap), 256, 0, (cudaStream_t)stream>>>(R, world, rank, lo4, hi4, lr, wd);
+  RS_CHECK_LAUNCH();
+  return RS_OK;
+}
+
+RS_API int rs_mark_rows(const rs_segments *seg, int64_t n, uint8_t *touched, int64_t rows, int32_t *status, void *stream) {
+  RS_CHECK_ARG(seg && seg->uniq && seg->n_uniq && touched, RS_E_ARG, "rs_mark_rows: null argument");
+  RS_CHECK_ARG(n > 0 && rows > 0, RS_E_SHAPE, "rs_mark_rows: bad n / rows");
+  int64_t blocks = (n + 255) / 256;
+  const int cap = rs::num_sms() * 8;
+  mark_rows_kernel<<<(int)(blocks < cap ? blocks : cap), 256, 0, (cudaStream_t)stream>>>(seg->uniq, seg->n_uniq, touched, rows, status);
+  RS_CHECK_LAUNCH();
+  return RS_OK;
+}
+
+RS_API int rs_replica_update(float *const *w, const float *const *g, const uint8_t *const *touched, int64_t numel, int32_t world,
+                             int32_t rank, const rs_update *u, void *stream) {
+  RS_CHECK_ARG(w && g && touched && u && world >= 1 && world <= RS_MAX_RANKS && rank >= 0 && rank < world, RS_E_ARG,
+               "rs_replica_update: bad argument");
+  RS_CHECK_ARG(u->mode == RS_UPD_SGD || u->mode == RS_UPD_ADAM, RS_E_UNSUPPORTED, "rs_replica_update: mode must be RS_UPD_SGD or RS_UPD_ADAM");
+  RS_CHECK_ARG(u->width >= 4 && u->width % 4 == 0 && numel >= 0 && numel % u->width == 0, RS_E_SHAPE,
+               "rs_replica_update: width must be a multiple of 4 that divides numel");
+  if (u->mode == RS_UPD_ADAM) RS_CHECK_ARG(u->step >= 1, RS_E_ARG, "rs_replica_update: Adam needs step >= 1");
+  Replicas R;
+  Flags T;
+  for (int k = 0; k < world; ++k) {
+    RS_CHECK_ARG(w[k] && g[k] && touched[k], RS_E_ARG, "rs_replica_update: null buffer for rank %d", k);
+    R.w[k] = w[k];
+    R.g[k] = g[k];
+    T.t[k] = touched[k];
+  }
+  int64_t lo4, hi4;
+  replica_slice(numel / 4, world, rank, lo4, hi4);
+  if (hi4 <= lo4) return RS_OK;
+  if (u->mode == RS_UPD_ADAM) RS_CHECK_ARG(u->m && u->v, RS_E_ARG, "rs_replica_update: Adam needs this rank's m and v slices");
+  rs::UpdParams P;
+  rs::set_opt_scalars(u, P);
+  int64_t blocks = (hi4 - lo4 + 255) / 256;
+  const int cap = rs::num_sms() * 8;
+  const int grid = (int)(blocks < cap ? blocks : cap);
+  cudaStream_t st = (cudaStream_t)stream;
+  if (u->mode == RS_UPD_SGD)
+    replica_update_kernel<RS_UPD_SGD><<<grid, 256, 0, st>>>(R, T, world, rank, lo4, hi4, u->width / 4, nullptr, nullptr, P.lr, P.wd,
+                                                            P.beta1, P.beta2, P.eps, P.step_size, P.inv_sqrt_bc2);
+  else
+    replica_update_kernel<RS_UPD_ADAM><<<grid, 256, 0, st>>>(R, T, world, rank, lo4, hi4, u->width / 4, u->m, u->v, P.lr, P.wd,
+                                                             P.beta1, P.beta2, P.eps, P.step_size, P.inv_sqrt_bc2);
   RS_CHECK_LAUNCH();
   return RS_OK;
 }

@@ -184,6 +184,10 @@ class _FieldModel(nn.Module):
                 ws.copy_(_xavier_concat(self.small_cards, width, row_dim, dev, (seed or 0) + 7919))     # same bits on every rank
                 self.weight_small = nn.Parameter(ws, requires_grad=False)
                 self.gsmall, self.gsmall_ptrs = fab.alloc((self.small_total, width), torch.float32, dev)
+                # rows of the small tables this rank's batch touched (lazy update with Adam or weight decay); allocated with
+                # the other symmetric buffers so that no step ever allocates collectively
+                self.touched_small, self.touched_ptrs = fab.alloc((self.small_total,), torch.uint8, dev)
+                self.adam_m_small = self.adam_v_small = None
                 self._big_cols_t = torch.tensor(big, dtype=torch.int64, device=dev)
                 self._small_cols_t = torch.tensor(small, dtype=torch.int64, device=dev)
                 add = [0] * self.F
@@ -222,20 +226,29 @@ class _FieldModel(nn.Module):
         if self.hybrid:
             self.weight_small.data.copy_(self._field_rows(gw, self.small_fields))
 
-    def assemble_global(self, shards):
+    def assemble_global(self, shards, small=None):
         """inverse of load_global (tests / verification): list of every rank's weight shard -> the full (total_rows, W) table
-        (the replicated fields are taken from this rank's copy)."""
+        (the replicated fields are taken from this rank's copy, or from `small`, a full (small_total, W) table).  The same
+        call assembles Adam's moments: pass every rank's adam_m and, as `small`, the ranks' adam_m_small slices concatenated
+        in rank order (see small_slice)."""
         from . import dist as rsdist
         big = rsdist.unshard_rows(list(shards))
         if not self.hybrid:
             return big
+        small = self.weight_small.data if small is None else small.reshape(self.small_total, self.width)
         out = torch.empty(self.total_rows, self.width, dtype=big.dtype, device=big.device)
         for k, f in enumerate(self.big_fields):
             out[self.offsets_host[f]:self.offsets_host[f] + self.cards[f]] = big[self.big_offsets_host[k]:self.big_offsets_host[k] + self.cards[f]]
         for k, f in enumerate(self.small_fields):
             out[self.offsets_host[f]:self.offsets_host[f] + self.cards[f]] = \
-                self.weight_small.data[self.small_offsets_host[k]:self.small_offsets_host[k] + self.cards[f]].to(big.device)
+                small[self.small_offsets_host[k]:self.small_offsets_host[k] + self.cards[f]].to(big.device)
         return out
+
+    @property
+    def small_slice(self):
+        """hybrid placement: (lo, hi), the elements of the flat replicated table whose update (and Adam moments,
+        adam_m_small / adam_v_small) this rank owns"""
+        return ops.replica_slice(self.small_total * self.width, self.exchange.world, self.exchange.rank)
 
     def tables(self):
         return ops.tables_from_concat(self.weight.data, self.offsets_host, self.cards)
@@ -360,9 +373,9 @@ class _FieldModel(nn.Module):
         return cross, rec
 
     def _apply_hybrid(self, opt, rec):
-        if opt.kind != "sgd" or opt.weight_decay != 0.0:
-            raise RuntimeError("replicated small tables (hybrid placement) are updated with plain SGD, weight_decay = 0; "
-                               "build the model with replicate_below=0 to row-shard every table instead")
+        # plain SGD without decay moves an untouched row by lr * 0: every element is stepped (rs_replica_sgd).  Otherwise the
+        # update is lazy, as on one GPU: each rank flags the rows its batch touched and only flagged rows step.
+        lazy = opt.kind != "sgd" or opt.weight_decay != 0.0
         ex, W = self.exchange, self.width
         plan = rec["plan"]
         ex.wait_plan(plan)                       # (before this step's first barrier on this stream)
@@ -380,6 +393,11 @@ class _FieldModel(nn.Module):
             self.gsmall.zero_()
             ops.segment_update(segs_s, ops.RS_UPD_GRAD, W, Fs, stash=rec["stash_small"], scale=g, dense_grad=self.gsmall, tag="/small",
                                half_sm=True)
+            if lazy:
+                # peers read these flags only after finish_push's barrier, and the barrier that ends the step orders those
+                # reads before this zeroing in the next step (the discipline gsmall follows)
+                self.touched_small.zero_()
+                ops.mark_rows(segs_s, self.touched_small, self.small_total)
             small_done = torch.cuda.Event()
             small_done.record()
         # row-sharded tables: reduce per distinct row, store straight into the owners' buffers
@@ -388,7 +406,16 @@ class _FieldModel(nn.Module):
         ops.segment_update(segs_b, ops.RS_UPD_GRAD, W, Fb, grad_routes=routes, stash=rec["stash_big"], scale=g, tag="/push", half_sm=True)
         cur.wait_event(small_done)
         recv = ex.finish_push(plan, ent)         # barrier: pushed rows have landed, every rank's dense gradient is complete
-        ops.replica_sgd(self.small_ptrs, self.gsmall_ptrs, self.small_total * W, ex.world, ex.rank, opt.lr)
+        if not lazy:
+            ops.replica_sgd(self.small_ptrs, self.gsmall_ptrs, self.small_total * W, ex.world, ex.rank, opt.lr)
+        else:
+            if opt.kind == "adam" and self.adam_m_small is None:
+                lo, hi = self.small_slice
+                self.adam_m_small = torch.zeros(hi - lo, dtype=torch.float32, device=g.device)
+                self.adam_v_small = torch.zeros(hi - lo, dtype=torch.float32, device=g.device)
+            ops.replica_update(self.small_ptrs, self.gsmall_ptrs, self.touched_ptrs, self.small_total * W, W, ex.world, ex.rank,
+                               opt.kind, opt.lr, opt.weight_decay, m=self.adam_m_small, v=self.adam_v_small, betas=opt.betas,
+                               eps=opt.eps, step=opt.step_count)
         osegs = ex.owner_segments(plan, self.weight.shape[0], W)
         self._row_update(opt, osegs, 1, tag="/owner", dense=recv)
         from .dist import _phase

@@ -600,6 +600,54 @@ def replica_sgd(w_ptrs, g_ptrs, numel, world, rank, lr, wd=0.0):
     _count()
 
 
+def replica_slice(numel, world, rank):
+    """(lo, hi) in floats of the elements rank `rank` updates in replica_sgd / replica_update (float4 slices,
+    per = ceil(numel / 4 / world))"""
+    n4 = int(numel) // 4
+    per = (n4 + world - 1) // world
+    lo4 = min(per * rank, n4)
+    return lo4 * 4, min(lo4 + per, n4) * 4
+
+
+def mark_rows(segs, touched, rows):
+    """touched[uniq[j]] = 1 for the distinct rows of a finished sort (rs_mark_rows; the count stays on the device).
+    touched: uint8 (rows,), zeroed by the caller."""
+    _need_cuda(touched)
+    if touched.dtype != torch.uint8 or not touched.is_contiguous() or touched.numel() < rows:
+        raise ValueError("touched must be a contiguous uint8 tensor of at least `rows` flags")
+    with _timed("mark_rows"):
+        _lib.check(_lib.load().rs_mark_rows(C.byref(segs.seg), segs.n, touched.data_ptr(), int(rows),
+                                            status_word(touched.device).data_ptr(), _stream()), "rs_mark_rows")
+    _count()
+
+
+def replica_update(w_ptrs, g_ptrs, flag_ptrs, numel, width, world, rank, kind, lr, wd=0.0, m=None, v=None, betas=(0.9, 0.999),
+                   eps=1e-8, step=1):
+    """Replicated table, lazy row update (rs_replica_update): rows flagged by some rank (flag_ptrs: every rank's uint8
+    touched array) take an SGD ("sgd") or Adam ("adam") step on the rank-ordered sum of the ranks' gradients, stored into
+    every rank's copy; the others keep their bits.  m / v: this rank's moment slices, replica_slice() floats from its lo.
+    Barriers before and after are the caller's."""
+    if kind not in ("sgd", "adam"):
+        raise ValueError("kind must be 'sgd' or 'adam'")
+    u = _lib.rs_update()
+    u.mode, u.width = (RS_UPD_SGD if kind == "sgd" else RS_UPD_ADAM), int(width)
+    if kind == "adam":
+        lo, hi = replica_slice(numel, world, rank)
+        for name, t in (("m", m), ("v", v)):
+            if t is None or t.dtype != torch.float32 or not t.is_contiguous() or t.numel() != hi - lo:
+                raise ValueError(f"{name} must be a contiguous float32 slice of {hi - lo} elements")
+            if hi > lo:
+                _need_cuda(t)
+                setattr(u, name, t.data_ptr())
+    u.lr, u.wd, u.beta1, u.beta2, u.eps, u.step = lr, wd, betas[0], betas[1], eps, step
+    W = (C.c_void_p * world)(*[int(p) for p in w_ptrs])
+    G = (C.c_void_p * world)(*[int(p) for p in g_ptrs])
+    T = (C.c_void_p * world)(*[int(p) for p in flag_ptrs])
+    with _timed(f"replica_update[{kind}]"):
+        _lib.check(_lib.load().rs_replica_update(W, G, T, int(numel), world, rank, C.byref(u), _stream()), "rs_replica_update")
+    _count()
+
+
 def adam_dense(p, g, m, v, step, lr=1e-3, wd=0.0, betas=(0.9, 0.999), eps=1e-8):
     _need_cuda(p, g, m, v)
     _lib.check(_lib.load().rs_adam_dense(p.data_ptr(), g.data_ptr(), m.data_ptr(), v.data_ptr(), p.numel(), lr, wd, betas[0],

@@ -21,7 +21,12 @@ class FusedRowOptimizer:
     summed gradient, as ``torch.optim`` steps once on the accumulated ``.grad``: the moments advance once and the decay
     term is applied once.  Plain SGD without decay applies the forwards one after another (the same result up to
     rounding).  A row-sharded table takes one forward per step with Adam or weight decay (several raise), and so does
-    the stash-free FFM forward (``RS_FFM_RECOMPUTE=1``) with weight decay."""
+    the stash-free FFM forward (``RS_FFM_RECOMPUTE=1``) with weight decay.
+
+    Multi-GPU: row-sharded tables are stepped by their owners; the replicated small tables of the hybrid placement are
+    stepped by rs_replica_update, which updates only rows some rank's batch touched (lazy, as on one GPU) and keeps each
+    rank's slice of the Adam moments (``adam_m_small`` / ``adam_v_small``, bounds ``small_slice``).  Plain SGD without
+    decay there steps every element with rs_replica_sgd (an untouched row's gradient is zero)."""
 
     def __init__(self, model, dense_optimizer=None, lr=0.01, kind="sgd", weight_decay=0.0, betas=(0.9, 0.999), eps=1e-8,
                  data_parallel=True):

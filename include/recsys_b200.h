@@ -292,6 +292,27 @@ int rs_shard_serve(const rs_shard *S, const float *table, int64_t rows, int32_t 
  * precede (all g complete) and follow (before g or w are touched again) the call. */
 int rs_replica_sgd(float *const *w, const float *const *g, int64_t numel, int32_t world, int32_t rank, float lr, float wd,
                    void *stream);
+/* Replicated small tables with the LAZY row update (weight decay and/or Adam): only rows that some rank's batch touched
+ * step, as in rs_segment_update; the others keep their bits (w, m and v).
+ *   rs_mark_rows       touched[uniq[j]] = 1 for j < *seg->n_uniq (read on the device; `n` = the sort's lookup count only
+ *                      sizes the grid).  touched: this rank's own uint8 array of `rows` flags in symmetric memory, zeroed
+ *                      by the caller on the stream beforehand.  Ranks never write each other's flags.
+ *   rs_replica_update  rank `rank` owns the float4 slice [lo4, hi4) of n4 = numel / 4, per = ceil(n4 / world),
+ *                      lo4 = min(rank * per, n4), hi4 = min(lo4 + per, n4) -- rs_replica_sgd's slices.  For each float4 i
+ *                      of row i * 4 / width (width % 4 == 0, so a float4 never straddles rows; a slice may split a row) it
+ *                      ORs the `world` flags touched[r][row]; an untouched element is skipped (no load, no store).
+ *                      Otherwise the `world` gradients g[r] are added in rank order (rs_replica_sgd's sum), u->mode
+ *                      (RS_UPD_SGD or RS_UPD_ADAM; others are refused) is applied with rs_segment_update's arithmetic and
+ *                      bias correction (u->lr, wd, beta1, beta2, eps, step), and w is stored into every replica.  The
+ *                      flags decide, not the gradient: a touched row whose summed gradient is exactly zero still steps.
+ *                      Adam's moments are NOT replicated: u->m / u->v point at this rank's slice only ((hi4 - lo4) * 4
+ *                      floats, element 0 = element lo4 * 4 of the table); u->width = row width.
+ * Barriers: every rank's g and flags must be complete before any rank calls rs_replica_update (the barrier after the
+ * gradient reduce), and a cross-rank barrier must follow it before any rank zeroes its flags or gradient, or touches w,
+ * again. */
+int rs_mark_rows(const rs_segments *seg, int64_t n, uint8_t *touched, int64_t rows, int32_t *status, void *stream);
+int rs_replica_update(float *const *w, const float *const *g, const uint8_t *const *touched, int64_t numel, int32_t world,
+                      int32_t rank, const rs_update *u, void *stream);
 
 /* Fused DENSE Adam sweep with torch.optim.Adam's exact arithmetic order ("reference-Adam" mode for the
  * MovieLens-sized tables; scripts/deepfm.py:55). */
