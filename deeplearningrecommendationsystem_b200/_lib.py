@@ -148,6 +148,8 @@ SIGNATURES = {
     "rs_gemm_nt_3xtf32": [_PP(rs_gemm_nt), _P],
     "rs_gru_fwd": [_P, _L, _I, _I, _P, _P, _P, _P, _P],
     "rs_gru_bwd": [_P, _P, _P, _P, _P, _L, _I, _I, _P, _P, _P],
+    "rs_augru_fwd": [_P, _P, _L, _I, _I, _P, _P, _P, _P, _P],
+    "rs_augru_bwd": [_P, _P, _P, _P, _P, _P, _L, _I, _I, _P, _P, _P, _P],
 }
 
 _lib = None

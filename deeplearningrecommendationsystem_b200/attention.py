@@ -1,4 +1,4 @@
-"""Attention pooling (AFM), target attention (DIN / DIEN) and the GRU recurrence of the drop-in modules."""
+"""Attention pooling (AFM), target attention (DIN / DIEN) and the GRU / AUGRU recurrences of the drop-in modules."""
 import torch
 
 
@@ -64,6 +64,13 @@ def din_attention(rows, unit, pool):
     return _DINAttention.apply(rows.contiguous(), pool, l0.weight, l0.bias, l1.weight, l1.bias, l2.weight, l2.bias)
 
 
+def din_attention_weights(rows, unit):
+    """The softmax weights w (B, L) of din_attention themselves (the DIEN paper's attention scores), bit-identical to the
+    weights the pooling and scaling modes apply; the gradient with respect to w flows back through the unit into rows."""
+    from . import ops
+    return din_attention(rows, unit, ops.DIN_WEIGHTS)
+
+
 class _GRURecurrence(torch.autograd.Function):
     """L sequential GRU steps on precomputed input projections (rs_gru_fwd / rs_gru_bwd).  Returns h_L (B, H)."""
 
@@ -87,11 +94,49 @@ class _GRURecurrence(torch.autograd.Function):
         return d_gi, flat.t() @ h_prev.reshape(B * L, H), flat.sum(dim=0)
 
 
+def _check_gru(gru, name):
+    if gru.num_layers != 1 or gru.bidirectional or not gru.batch_first or gru.hidden_size not in (8, 16, 32, 64):
+        raise NotImplementedError(f"{name}: single-layer batch_first GRU with hidden size in {{8,16,32,64}}")
+
+
 def gru_last_hidden(x, gru):
     """hidden[-1] of a single-layer batch_first GRU started from zeros                  reference model/dien.py:61-64.
     Input projection = one library GEMM; the recurrence and its BPTT run in the hand-written kernels."""
-    H = gru.hidden_size
-    if gru.num_layers != 1 or gru.bidirectional or not gru.batch_first or H not in (8, 16, 32, 64):
-        raise NotImplementedError("gru_last_hidden: single-layer batch_first GRU with hidden size in {8,16,32,64}")
+    _check_gru(gru, "gru_last_hidden")
     gi = torch.nn.functional.linear(x, gru.weight_ih_l0, gru.bias_ih_l0)
     return _GRURecurrence.apply(gi, gru.weight_hh_l0, gru.bias_hh_l0)
+
+
+class _AUGRURecurrence(torch.autograd.Function):
+    """L sequential AUGRU steps on precomputed input projections (rs_augru_fwd / rs_augru_bwd).  Returns h_L (B, H)."""
+
+    @staticmethod
+    def forward(ctx, gi, att, w_hh, b_hh):
+        from . import ops
+        need = any(ctx.needs_input_grad)
+        h_all, gates = ops.augru_fwd(gi, att, w_hh.detach(), b_hh.detach(), want_gates=need)
+        if need:
+            ctx.save_for_backward(att, w_hh, h_all, gates)
+        return h_all[:, -1].clone()
+
+    @staticmethod
+    def backward(ctx, g_last):
+        from . import ops
+        att, w_hh, h_all, gates = ctx.saved_tensors
+        B, L, H = h_all.shape
+        d_gi, d_gh, d_att = ops.augru_bwd(w_hh.detach(), att, h_all, gates, g_h_last=g_last.contiguous())
+        h_prev = torch.cat([torch.zeros(B, 1, H, device=h_all.device), h_all[:, :-1]], dim=1)
+        flat = d_gh.view(B * L, 3 * H)
+        return d_gi, d_att, flat.t() @ h_prev.reshape(B * L, H), flat.sum(dim=0)
+
+
+def augru_last_hidden(x, att, gru):
+    """h_L of the DIEN paper's attention-gated GRU (AUGRU) with the weights of `gru` (an nn.GRU), h0 = 0:
+    u = att[:, t] (1 - z),  h_t = (1 - u) h_{t-1} + u n  with torch's gates r, z, n.  x (B, L, D) is NOT scaled by att;
+    att (B, L) gates the update instead.  att == 1 gives gru_last_hidden, att == 0 gives zeros.
+    Input projection = one library GEMM; the recurrence and its BPTT (including d att) run in the hand-written kernels."""
+    _check_gru(gru, "augru_last_hidden")
+    if att.dim() != 2 or tuple(att.shape) != tuple(x.shape[:2]):
+        raise ValueError(f"augru_last_hidden: att has shape {tuple(att.shape)}, expected {tuple(x.shape[:2])}")
+    gi = torch.nn.functional.linear(x, gru.weight_ih_l0, gru.bias_ih_l0)
+    return _AUGRURecurrence.apply(gi, att.contiguous(), gru.weight_hh_l0, gru.bias_hh_l0)

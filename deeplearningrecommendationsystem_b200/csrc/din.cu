@@ -1,7 +1,7 @@
 // DIN target attention, forward and backward (reference model/din.py:39-47; model/dien.py:27-37 with pool == 0).
 //
 //   z_l = [h_l, h_l - t, t];  a1 = relu(W0 z_l + b0);  a2 = relu(W1 a1 + b1);  s_l = W2 a2 + b2
-//   w = softmax_l(s)  (no mask, no scaling);  out = sum_l w_l h_l  (pool)   or   out_l = w_l h_l  (scale)
+//   w = softmax_l(s)  (no mask, no scaling);  out = sum_l w_l h_l  (pool),  out_l = w_l h_l  (scale)  or  out = w  (weights)
 //
 // The (B, L, 3D) concat never exists: with W0 = [Wa | Wb | Wc],  W0 z_l = (Wa + Wb) h_l + (Wc - Wb) t, so the
 // target part is computed once per sample and the per-position part costs D*H1 instead of 3D*H1 MACs.
@@ -20,11 +20,11 @@ struct DinParams {
   const float *rows;  // (B, L+1, D): L history rows then the target row
   const float *W0, *b0, *W1, *b1, *W2, *b2;
   float *out, *attw;             // forward
-  const float *g_out;            // backward: (B, D) pool or (B, L, D) scale
+  const float *g_out;            // backward: (B, D) pool, (B, L, D) scale or (B, L) weights
   float *d_rows;                 // (B, L+1, D) gradient through the attention only
   float *dWab_p, *dWt_p, *dW1_p, *db0_p, *db1_p, *dW2_p, *db2_p;  // per-CTA partials
   int64_t B;
-  int L, pool;
+  int L, pool;                   // pool: RS_DIN_SCALE, RS_DIN_WEIGHTS, any other value pools
 };
 
 template <int D, int H1, int H2>
@@ -192,7 +192,9 @@ __global__ void __launch_bounds__(NT, 1) din_fwd_kernel(const __grid_constant__ 
     const int tid = threadIdx.x;
     if (P.attw)
       for (int l = tid; l < L; l += NT) P.attw[b * L + l] = w[l];
-    if (P.pool) {
+    if (P.pool == RS_DIN_WEIGHTS) {
+      for (int l = tid; l < L; l += NT) P.out[b * L + l] = w[l];
+    } else if (P.pool) {
       for (int d = tid; d < D; d += NT) {
         float acc = 0.f;
         for (int l = 0; l < L; ++l) acc = fmaf(w[l], h[l * D + d], acc);
@@ -228,8 +230,10 @@ __global__ void __launch_bounds__(NT, 1) din_bwd_kernel(const __grid_constant__ 
   __syncthreads();
   for (int64_t b = blockIdx.x; b < P.B; b += gridDim.x) {
     forward_sample<D, H1, H2>(P, sm, h, a1, a2, s, w, b);
-    // B1: dw[l] = <g_l, h_l>
-    {
+    // B1: dw[l] = <g_l, h_l>, or g_l itself when the weights are the output
+    if (P.pool == RS_DIN_WEIGHTS) {
+      for (int l = tid; l < L; l += NT) dw[l] = P.g_out[b * L + l];
+    } else {
       const int lane = tid & 31, warp = tid >> 5;
       for (int l = warp; l < L; l += NT / 32) {
         const float *g = P.pool ? P.g_out + b * D : P.g_out + (b * L + l) * (int64_t)D;
@@ -336,17 +340,27 @@ __global__ void __launch_bounds__(NT, 1) din_bwd_kernel(const __grid_constant__ 
       }
     }
     __syncthreads();
-    // B8: d h[l][k] = w[l] g_l[k] + sum_j da1[l][j] (Wa+Wb)[j][k];  d target = dt
+    // B8: d h[l][k] = w[l] g_l[k] + sum_j da1[l][j] (Wa+Wb)[j][k];  d target = dt.  The weights output has no direct
+    // path w[l] g_l: its gradient reaches the rows through the MLP only.
     {
       float *o = P.d_rows + b * (int64_t)(L + 1) * D;
-      for (int e = tid; e < L * D; e += NT) {
-        const int l = e / D, k = e - l * D;
-        const float g = P.pool ? P.g_out[b * D + k] : P.g_out[(b * L + l) * (int64_t)D + k];
-        float acc = w[l] * g;
+      auto chain = [&](int l, int k, float acc) {
         const float *da = a1 + l * H1;
 #pragma unroll 8
         for (int j = 0; j < H1; ++j) acc = fmaf(da[j], sm[Y::WAB + j * (D + 1) + k], acc);
-        o[e] = acc;
+        return acc;
+      };
+      if (P.pool == RS_DIN_WEIGHTS) {
+        for (int e = tid; e < L * D; e += NT) {
+          const int l = e / D, k = e - l * D;
+          o[e] = chain(l, k, 0.f);
+        }
+      } else {
+        for (int e = tid; e < L * D; e += NT) {
+          const int l = e / D, k = e - l * D;
+          const float g = P.pool ? P.g_out[b * D + k] : P.g_out[(b * L + l) * (int64_t)D + k];
+          o[e] = chain(l, k, w[l] * g);
+        }
       }
       for (int k = tid; k < D; k += NT) o[(int64_t)L * D + k] = sm[Y::DT + k];
     }

@@ -10,7 +10,8 @@
 //             while the next 32 columns are being read back.               MMA: M=128, N=H2, K=H1 -> TMEM cols [H1, H1+H2)
 //   layer 2   w2 . relu(.) + b2                a per-row dot product in the final epilogue.
 // All weights stay resident in shared memory as tf32 hi/lo pairs (3xTF32: lo*hi + hi*lo + hi*hi, ~1e-6 relative) in
-// the canonical K-major core-matrix layout.  The softmax over L and the weighted sum run in din_softmax_pool_kernel.
+// the canonical K-major core-matrix layout.  The softmax over L and the weighted sum run in din_softmax_pool_kernel;
+// with pool == RS_DIN_WEIGHTS the softmax weights are the output and nothing is scaled or pooled.
 #include "common.cuh"
 #include "tc.cuh"
 
@@ -277,6 +278,7 @@ __global__ void __launch_bounds__(256) din_softmax_pool_kernel(const float *__re
     const float inv = 1.f / sum;
     float *w = attw + b * L;
     for (int l = lane; l < L; l += 32) w[l] = expf(s[l] - mx) * inv;
+    if (pool == RS_DIN_WEIGHTS) continue;   // attw is the output
     __syncwarp();
     const float *h = rows + b * (int64_t)(L + 1) * D;
     if (pool) {
@@ -300,7 +302,8 @@ __global__ void __launch_bounds__(256) din_softmax_pool_kernel(const float *__re
 }
 
 // ---------------------------------------------------------------------------------------------------- backward
-// ds[b][l] = d loss / d score: softmax backward of  out = sum_l w_l h_l  (pool)  or  out_l = w_l h_l.  Warp per sample.
+// ds[b][l] = d loss / d score: softmax backward of  out = sum_l w_l h_l  (pool),  out_l = w_l h_l  or  out = w  (weights,
+// g_out (B, L) = d loss / d w).  Warp per sample.
 __global__ void __launch_bounds__(256) din_dscore_kernel(const float *__restrict__ rows, const float *__restrict__ attw,
                                                          const float *__restrict__ g_out, int64_t B, int L, int D, int pool,
                                                          float *__restrict__ ds) {
@@ -313,18 +316,26 @@ __global__ void __launch_bounds__(256) din_dscore_kernel(const float *__restrict
     float *o = ds + b * L;
     // lane <-> history slot: dw_l = <g, h_l> from 16-byte loads (D / 4 independent loads per slot), no shuffles
     float tsum = 0.f;
-    for (int l = lane; l < L; l += 32) {
-      const float *g = pool ? g_out + b * D : g_out + (b * L + l) * (int64_t)D;
-      const float *hl = h + (int64_t)l * D;
-      float p0 = 0.f, p1 = 0.f;
-      for (int q = 0; q + 8 <= D; q += 8) {
-        p0 += rs::f4_dot(rs::ldg_f4(g + q), rs::ldg_nc_f4(hl + q));
-        p1 += rs::f4_dot(rs::ldg_f4(g + q + 4), rs::ldg_nc_f4(hl + q + 4));
+    if (pool == RS_DIN_WEIGHTS) {
+      for (int l = lane; l < L; l += 32) {
+        const float dw = g_out[b * L + l];
+        o[l] = dw;
+        tsum = fmaf(w[l], dw, tsum);
       }
-      if (D & 4) p0 += rs::f4_dot(rs::ldg_f4(g + (D & ~7)), rs::ldg_nc_f4(hl + (D & ~7)));
-      const float dw = p0 + p1;
-      o[l] = dw;
-      tsum = fmaf(w[l], dw, tsum);
+    } else {
+      for (int l = lane; l < L; l += 32) {
+        const float *g = pool ? g_out + b * D : g_out + (b * L + l) * (int64_t)D;
+        const float *hl = h + (int64_t)l * D;
+        float p0 = 0.f, p1 = 0.f;
+        for (int q = 0; q + 8 <= D; q += 8) {
+          p0 += rs::f4_dot(rs::ldg_f4(g + q), rs::ldg_nc_f4(hl + q));
+          p1 += rs::f4_dot(rs::ldg_f4(g + q + 4), rs::ldg_nc_f4(hl + q + 4));
+        }
+        if (D & 4) p0 += rs::f4_dot(rs::ldg_f4(g + (D & ~7)), rs::ldg_nc_f4(hl + (D & ~7)));
+        const float dw = p0 + p1;
+        o[l] = dw;
+        tsum = fmaf(w[l], dw, tsum);
+      }
     }
     tsum = rs::warp_sum(tsum);
     for (int l = lane; l < L; l += 32) o[l] = w[l] * (o[l] - tsum);   // each lane re-reads only what it wrote
@@ -347,7 +358,7 @@ struct DinTcBwdParams {
 //   da0 = dz1 W1                   MMA: M=128, N=H1, K=H2   (W1 resident as an (N=H1, K=H2) K-major image)
 //   dz0 = da0 [a0 > 0]             (epilogue -> written out, and straight into the next A operand)
 //   dx  = dz0 (Wa + Wb)            MMA: M=128, N=D,  K=H1   ((Wa+Wb) resident as (N=D, K=H1))
-//   d_rows[b, l] = dx + w_l g      (the direct path of the weighted sum)
+//   d_rows[b, l] = dx + w_l g      (the direct path of the weighted sum; none when the weights are the output)
 __global__ void __launch_bounds__(NTH, 1) din_bwd_tc_kernel(const __grid_constant__ DinTcBwdParams P) {
   extern __shared__ __align__(128) uint32_t sm[];
   __shared__ uint64_t bar[2];   // one per warpgroup: that group's operand buffer has been read by its MMAs
@@ -392,7 +403,8 @@ __global__ void __launch_bounds__(NTH, 1) din_bwd_tc_kernel(const __grid_constan
   const int64_t nrows = P.B * P.L;
   const int64_t ntiles = (nrows + MT - 1) / MT;
   const int64_t first_tile = (int64_t)blockIdx.x * 2 + grp, tile_step = (int64_t)gridDim.x * 2;   // the two warpgroups take alternate tiles
-  const int nG = (D + 31) / 32, nS = nchunkA + nchunkB + nG;   // stages of one tile: act1 chunks, act0 chunks, g pieces
+  const bool direct = P.pool != RS_DIN_WEIGHTS;
+  const int nG = direct ? (D + 31) / 32 : 0, nS = nchunkA + nchunkB + nG;   // stages of one tile: act1 chunks, act0 chunks, g pieces
   // Every stage consumes eight 16-byte pieces of one row of a global array.  They are fetched one stage AHEAD into
   // `pre` (across tile boundaries too), so the load latency hides behind the previous stage's repack and MMAs.
   float4 pre[KC / 4];
@@ -543,21 +555,35 @@ __global__ void __launch_bounds__(NTH, 1) din_bwd_tc_kernel(const __grid_constan
     }
     rs::mbar_wait(&bar[grp], (uses - 1) & 1u);   // accumulator complete: the latest commit covers every earlier MMA
     fence_after_sync();
-    // ---- d_rows[b, l] = dx + w_l g
-    const float wl = valid ? P.attw[r] : 0.f;
-    for (int c0 = 0; c0 < D; c0 += 32) {
-      advance();
-      uint32_t v[32];
-      tmem_ld32(tmem, warp, H1 + c0, v);
-      if (valid) {
+    // ---- d_rows[b, l] = dx + w_l g,  or dx alone in the weights mode (no g stages were fetched)
+    if (direct) {
+      const float wl = valid ? P.attw[r] : 0.f;
+      for (int c0 = 0; c0 < D; c0 += 32) {
+        advance();
+        uint32_t v[32];
+        tmem_ld32(tmem, warp, H1 + c0, v);
+        if (valid) {
 #pragma unroll
-        for (int q = 0; q < 8; ++q) {
-          if (c0 + 4 * q < D) {
-            const float4 g4 = cur[q];
-            rs::stg_f4(P.d_rows + rr * D + c0 + 4 * q,
-                       make_float4(fmaf(wl, g4.x, __uint_as_float(v[4 * q + 0])), fmaf(wl, g4.y, __uint_as_float(v[4 * q + 1])),
-                                   fmaf(wl, g4.z, __uint_as_float(v[4 * q + 2])), fmaf(wl, g4.w, __uint_as_float(v[4 * q + 3]))));
+          for (int q = 0; q < 8; ++q) {
+            if (c0 + 4 * q < D) {
+              const float4 g4 = cur[q];
+              rs::stg_f4(P.d_rows + rr * D + c0 + 4 * q,
+                         make_float4(fmaf(wl, g4.x, __uint_as_float(v[4 * q + 0])), fmaf(wl, g4.y, __uint_as_float(v[4 * q + 1])),
+                                     fmaf(wl, g4.z, __uint_as_float(v[4 * q + 2])), fmaf(wl, g4.w, __uint_as_float(v[4 * q + 3]))));
+            }
           }
+        }
+      }
+    } else {
+      for (int c0 = 0; c0 < D; c0 += 32) {
+        uint32_t v[32];
+        tmem_ld32(tmem, warp, H1 + c0, v);
+        if (valid) {
+#pragma unroll
+          for (int q = 0; q < 8; ++q)
+            if (c0 + 4 * q < D)
+              rs::stg_f4(P.d_rows + rr * D + c0 + 4 * q, make_float4(__uint_as_float(v[4 * q + 0]), __uint_as_float(v[4 * q + 1]),
+                                                                      __uint_as_float(v[4 * q + 2]), __uint_as_float(v[4 * q + 3])));
         }
       }
     }
@@ -614,11 +640,14 @@ RS_API int rs_din_fwd_tc(const float *rows, int64_t B, int32_t L, int32_t D, con
   const int64_t pairs = (ntiles + 1) / 2;   // a CTA's two warpgroups take alternate tiles
   din_score_tc_kernel<<<(unsigned)(pairs < sms ? pairs : sms), NTH, smem, st>>>(P);
   RS_CHECK_LAUNCH();
-  // attw doubles as the softmax output the backward needs; without it the scores are normalised in place
-  float *wout = attw ? attw : score;
+  // attw doubles as the softmax output the backward needs; without it the scores are normalised in place.  In the
+  // weights mode the output is that softmax output.
+  float *wout = pool == RS_DIN_WEIGHTS ? out : attw ? attw : score;
   int64_t blocks = (B + 7) / 8;
   din_softmax_pool_kernel<<<(unsigned)(blocks < 8 * sms ? blocks : 8 * sms), 256, 0, st>>>(rows, score, B, L, D, pool, out, wout);
   RS_CHECK_LAUNCH();
+  if (pool == RS_DIN_WEIGHTS && attw && attw != out)
+    RS_CUDA(cudaMemcpyAsync(attw, out, (size_t)B * L * sizeof(float), cudaMemcpyDeviceToDevice, st));
   return RS_OK;
 }
 

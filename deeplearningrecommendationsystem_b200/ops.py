@@ -764,6 +764,40 @@ def gru_bwd(w_hh, h_all, gates, g_h_all=None, g_h_last=None):
     return d_gi, d_gh
 
 
+def augru_fwd(gi, att, w_hh, b_hh, want_gates=True):
+    """Attention-gated GRU (DIEN's AUGRU): gi (B, L, 3H), att (B, L)  ->  h_all (B, L, H), gates (B, L, 4H) | None."""
+    gi, att, w_hh, b_hh = _f32(gi), _f32(att), _f32(w_hh), _f32(b_hh)
+    _need_cuda(gi, att, w_hh, b_hh)
+    B, L, H3 = gi.shape
+    H = H3 // 3
+    if tuple(att.shape) != (B, L):
+        raise ValueError(f"augru_fwd: att has shape {tuple(att.shape)}, expected {(B, L)}")
+    h_all = torch.empty(B, L, H, dtype=torch.float32, device=gi.device)
+    gates = torch.empty(B, L, 4 * H, dtype=torch.float32, device=gi.device) if want_gates else None
+    if B == 0:
+        return h_all, gates
+    with _timed("augru_fwd"):
+        _lib.check(_lib.load().rs_augru_fwd(gi.data_ptr(), att.data_ptr(), B, L, H, w_hh.data_ptr(), b_hh.data_ptr(), h_all.data_ptr(),
+                                            _p(gates), _stream()), "rs_augru_fwd")
+    _count()
+    return h_all, gates
+
+
+def augru_bwd(w_hh, att, h_all, gates, g_h_all=None, g_h_last=None):
+    """-> d_gi, d_gh (B, L, 3H), d_att (B, L)."""
+    B, L, H = h_all.shape
+    att, g_h_all, g_h_last = _f32(att), _f32(g_h_all), _f32(g_h_last)
+    d_gi = torch.empty(B, L, 3 * H, dtype=torch.float32, device=h_all.device)
+    d_gh = torch.empty_like(d_gi)
+    d_att = torch.empty(B, L, dtype=torch.float32, device=h_all.device)
+    with _timed("augru_bwd"):
+        _lib.check(_lib.load().rs_augru_bwd(_f32(w_hh).data_ptr(), att.data_ptr(), h_all.data_ptr(), gates.data_ptr(), _p(g_h_all),
+                                            _p(g_h_last), B, L, H, d_gi.data_ptr(), d_gh.data_ptr(), d_att.data_ptr(), _stream()),
+                   "rs_augru_bwd")
+    _count()
+    return d_gi, d_gh, d_att
+
+
 def afm_fwd(E, W, b, h, want_attw=True):
     """pooled (B, D), attw (B, P) | None."""
     E, W, b, h = _f32(E), _f32(W), _f32(b), _f32(h).reshape(-1)
@@ -853,8 +887,18 @@ def din_tc_supported(D, H1, H2):
     return D in (16, 32, 64) and H1 in (64, 128) and H2 in (32, 64)
 
 
+DIN_WEIGHTS = "weights"        # `pool` value of din_fwd / din_bwd / din_bwd_tc: the softmax weights (B, L) are the output
+
+
+def _din_mode(pool):
+    """the rs_din_* `pool` argument: RS_DIN_WEIGHTS (2) for DIN_WEIGHTS, else RS_DIN_POOL (1) / RS_DIN_SCALE (0) by truth"""
+    return 2 if isinstance(pool, str) and pool == DIN_WEIGHTS else int(bool(pool))
+
+
 def din_fwd(rows, ws, pool, want_attw=False, impl="auto", want_stash=False):
     """rows (B, L+1, D) = [history | target]; ws = (W0, b0, W1, b1, W2, b2) -> out (B,D) | (B,L,D), attw (B,L) | None.
+    pool: true -> (B, D) weighted sum, false -> (B, L, D) scaled history, DIN_WEIGHTS -> (B, L) softmax weights (then
+    attw, when wanted, is that same tensor).
 
     impl: "tc" = hidden layers on the tcgen05 tensor cores (rs_din_fwd_tc), "fused" = the CUDA-core kernel
     (rs_din_fwd), "auto" = tc when the shape is built and there are enough rows to fill the SMs (RS_DIN_TC=0 forces
@@ -865,13 +909,18 @@ def din_fwd(rows, ws, pool, want_attw=False, impl="auto", want_stash=False):
     B, L1, D = rows.shape
     L = L1 - 1
     w, keep = _din_weights(ws)
-    out = torch.empty((B, D) if pool else (B, L, D), dtype=torch.float32, device=rows.device)
+    mode = _din_mode(pool)
+    out = torch.empty((B, L) if mode == 2 else (B, D) if mode else (B, L, D), dtype=torch.float32, device=rows.device)
     if impl == "auto":
         fused_ok = D in (16, 32, 64) and (w.H1, w.H2) in ((128, 64), (64, 32))
         big = B * L >= DIN_TC_MIN_ROWS and os.environ.get("RS_DIN_TC", "1") != "0"
         impl = "tc" if din_tc_supported(D, w.H1, w.H2) and (big or not fused_ok) else "fused"
     stash_tc = want_stash and impl == "tc"
-    attw = torch.empty(B, L, dtype=torch.float32, device=rows.device) if (want_attw or stash_tc) else None
+    if mode == 2:
+        attw = out if (want_attw or stash_tc) else None
+    else:
+        attw = torch.empty(B, L, dtype=torch.float32, device=rows.device) if (want_attw or stash_tc) else None
+    kattw = None if mode == 2 else attw      # the weights mode writes its weights to `out` only
     if B == 0:
         return (out, attw, None) if want_stash else (out, attw)
     lib = _lib.load()
@@ -882,12 +931,12 @@ def din_fwd(rows, ws, pool, want_attw=False, impl="auto", want_stash=False):
         act0 = torch.empty(B * L, w.H1, dtype=torch.float32, device=rows.device) if stash_tc else None
         act1 = torch.empty(B * L, w.H2, dtype=torch.float32, device=rows.device) if stash_tc else None
         with _timed("din_fwd_tc"):
-            _lib.check(lib.rs_din_fwd_tc(rows.data_ptr(), B, L, D, C.byref(w), int(bool(pool)), out.data_ptr(), _p(attw), _p(act0),
+            _lib.check(lib.rs_din_fwd_tc(rows.data_ptr(), B, L, D, C.byref(w), mode, out.data_ptr(), _p(kattw), _p(act0),
                                          _p(act1), scratch.data_ptr(), nbytes.value, _stream()), "rs_din_fwd_tc")
         _count(3)
         return (out, attw, (attw, act0, act1) if stash_tc else None) if want_stash else (out, attw)
     with _timed("din_fwd"):
-        _lib.check(lib.rs_din_fwd(rows.data_ptr(), B, L, D, C.byref(w), int(bool(pool)), out.data_ptr(), _p(attw), _stream()),
+        _lib.check(lib.rs_din_fwd(rows.data_ptr(), B, L, D, C.byref(w), mode, out.data_ptr(), _p(kattw), _stream()),
                    "rs_din_fwd")
     _count()
     return (out, attw, None) if want_stash else (out, attw)
@@ -910,7 +959,7 @@ def din_bwd_tc(rows, ws, pool, g_out, stash):
     dz1 = torch.empty(B * L, H2, dtype=torch.float32, device=dev)
     ds = torch.empty(B, L, dtype=torch.float32, device=dev)
     with _timed("din_bwd_tc"):
-        _lib.check(_lib.load().rs_din_bwd_tc(rows.data_ptr(), B, L, D, C.byref(w), int(bool(pool)), g_out.data_ptr(), attw.data_ptr(),
+        _lib.check(_lib.load().rs_din_bwd_tc(rows.data_ptr(), B, L, D, C.byref(w), _din_mode(pool), g_out.data_ptr(), attw.data_ptr(),
                                              act0.data_ptr(), act1.data_ptr(), d_rows.data_ptr(), dz0.data_ptr(), dz1.data_ptr(),
                                              ds.data_ptr(), _stream()), "rs_din_bwd_tc")
     _count(2)
@@ -943,7 +992,7 @@ def din_bwd(rows, ws, pool, g_out):
     mk = lambda *shape: torch.empty(n, *shape, dtype=torch.float32, device=dev)   # noqa: E731
     dWab, dWt, dW1, db0, db1, dW2, db2 = mk(H1, D), mk(H1, D), mk(H2, H1), mk(H1), mk(H2), mk(H2), mk()
     with _timed("din_bwd"):
-        _lib.check(lib.rs_din_bwd(rows.data_ptr(), B, L, D, C.byref(w), int(bool(pool)), g_out.data_ptr(), d_rows.data_ptr(),
+        _lib.check(lib.rs_din_bwd(rows.data_ptr(), B, L, D, C.byref(w), _din_mode(pool), g_out.data_ptr(), d_rows.data_ptr(),
                                   dWab.data_ptr(), dWt.data_ptr(), dW1.data_ptr(), db0.data_ptr(), db1.data_ptr(), dW2.data_ptr(),
                                   db2.data_ptr(), n, _stream()), "rs_din_bwd")
     _count()

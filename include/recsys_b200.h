@@ -364,13 +364,18 @@ int rs_afm_bwd_tc(const float *E, int64_t B, int32_t F, int32_t D, int32_t A, co
 /* ---- DIN target attention (model/din.py:39-47; model/dien.py:27-37 with pool == 0), forward and backward.
  * rows (B, L+1, D): the L gathered history rows followed by the target row (the layout rs_gather_rows produces for
  * ids = [hist | target]).  Attention unit 3D -> H1 -> H2 -> 1 with ReLU (torch Linear layout (out, in)), softmax over
- * L without mask or scaling.  pool != 0: out (B, D) = sum_l w_l h_l;  pool == 0: out (B, L, D) = w_l h_l.
+ * L without mask or scaling.  `pool` selects the output:
+ *   RS_DIN_SCALE    out (B, L, D) = w_l h_l
+ *   RS_DIN_POOL     out (B, D) = sum_l w_l h_l          (every value other than RS_DIN_SCALE and RS_DIN_WEIGHTS pools)
+ *   RS_DIN_WEIGHTS  out (B, L) = w, bit-identical to the attw output of the other modes; nothing is scaled or pooled.
+ *                   The backward takes g_out (B, L) = d loss / d w, and d_rows carries only the chain through the MLP.
  * The concat [h, h-t, t] is never built: W0 z = (Wa+Wb) h + (Wc-Wb) t.  Built for D in {16,32,64} and
  * (H1,H2) in {(128,64),(64,32)}.
  * Backward recomputes the activations; d_rows (B, L+1, D) is the gradient THROUGH the attention (add the direct uses
  * of the rows outside).  Weight gradients come back as per-CTA partials (num_parts = rs_din_num_parts(B)), to be
  * added in index order:  dW0 = [dWab | dWab - dWt | dWt]  with dWab, dWt (parts, H1, D);  dW1 (parts, H2, H1);
  * db0 (parts, H1); db1 (parts, H2); dW2 (parts, H2); db2 (parts). */
+enum { RS_DIN_SCALE = 0, RS_DIN_POOL = 1, RS_DIN_WEIGHTS = 2 };
 typedef struct rs_din_weights {
   const float *W0, *b0, *W1, *b1, *W2, *b2;
   int32_t H1, H2;
@@ -411,6 +416,15 @@ int rs_gru_fwd(const float *gi, int64_t B, int32_t L, int32_t H, const float *w_
                float *gates, void *stream);
 int rs_gru_bwd(const float *w_hh, const float *h_all, const float *gates, const float *g_h_all, const float *g_h_last,
                int64_t B, int32_t L, int32_t H, float *d_gi, float *d_gh, void *stream);
+/* Attention-gated GRU of the DIEN paper (AUGRU), same conventions as rs_gru_*: with a_t = att[b, t] (B, L) and torch's
+ * gates r, z, n,   u = a_t (1 - z),  h_t = (1 - u) h_{t-1} + u n   (att == 1: nn.GRU; att == 0: h == 0).
+ * gates keeps the rs_gru_fwd layout (NULL for inference).  rs_augru_bwd also writes d_att (B, L), each entry a sum
+ * over H in a fixed order (bit-reproducible).  The CTA's 16 x L block of att is staged in shared memory, which bounds
+ * L (L <= 2352 at H = 64, 3552 at H = 8; RS_E_UNSUPPORTED beyond). */
+int rs_augru_fwd(const float *gi, const float *att, int64_t B, int32_t L, int32_t H, const float *w_hh, const float *b_hh,
+                 float *h_all, float *gates, void *stream);
+int rs_augru_bwd(const float *w_hh, const float *att, const float *h_all, const float *gates, const float *g_h_all,
+                 const float *g_h_last, int64_t B, int32_t L, int32_t H, float *d_gi, float *d_gh, float *d_att, void *stream);
 
 /* ---- C (M, N) = A^T B for row-major A (K, M), B (K, N): PNN "out" mode's batch-collapsed outer product
  * p = S^T S, S = sum_f e_f (model/pnn.py:69-72), on tcgen05 tensor cores with a 3xTF32 operand split (hi/lo) and fp32
