@@ -150,6 +150,9 @@ SIGNATURES = {
     "rs_gru_bwd": [_P, _P, _P, _P, _P, _L, _I, _I, _P, _P, _P],
     "rs_augru_fwd": [_P, _P, _L, _I, _I, _P, _P, _P, _P, _P],
     "rs_augru_bwd": [_P, _P, _P, _P, _P, _P, _L, _I, _I, _P, _P, _P, _P],
+    "rs_dien_negatives": [_P, _L, _I, _L, C.c_uint64, _P, _P, _P, _P],
+    "rs_dien_aux_fwd": [_P, _L, _P, _L, _P, _L, _L, _I, _I, _P, _P, _P, _P],
+    "rs_dien_aux_bwd": [_P, _L, _P, _L, _P, _L, _L, _I, _I, _P, _P, _P, _P, _P, _P],
 }
 
 _lib = None

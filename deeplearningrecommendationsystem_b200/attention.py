@@ -1,4 +1,5 @@
-"""Attention pooling (AFM), target attention (DIN / DIEN) and the GRU / AUGRU recurrences of the drop-in modules."""
+"""Attention pooling (AFM), target attention (DIN / DIEN), the GRU / AUGRU recurrences and DIEN's auxiliary loss of the
+drop-in modules."""
 import torch
 
 
@@ -94,6 +95,29 @@ class _GRURecurrence(torch.autograd.Function):
         return d_gi, flat.t() @ h_prev.reshape(B * L, H), flat.sum(dim=0)
 
 
+class _GRUSequence(torch.autograd.Function):
+    """_GRURecurrence returning every h_t (B, L, H); the backward runs rs_gru_bwd from the per-step gradient g_h_all."""
+
+    @staticmethod
+    def forward(ctx, gi, w_hh, b_hh):
+        from . import ops
+        need = any(ctx.needs_input_grad)
+        h_all, gates = ops.gru_fwd(gi, w_hh.detach(), b_hh.detach(), want_gates=need)
+        if need:
+            ctx.save_for_backward(w_hh, h_all, gates)
+        return h_all
+
+    @staticmethod
+    def backward(ctx, g_all):
+        from . import ops
+        w_hh, h_all, gates = ctx.saved_tensors
+        B, L, H = h_all.shape
+        d_gi, d_gh = ops.gru_bwd(w_hh.detach(), h_all, gates, g_h_all=g_all.contiguous())
+        h_prev = torch.cat([torch.zeros(B, 1, H, device=h_all.device), h_all[:, :-1]], dim=1)
+        flat = d_gh.view(B * L, 3 * H)
+        return d_gi, flat.t() @ h_prev.reshape(B * L, H), flat.sum(dim=0)
+
+
 def _check_gru(gru, name):
     if gru.num_layers != 1 or gru.bidirectional or not gru.batch_first or gru.hidden_size not in (8, 16, 32, 64):
         raise NotImplementedError(f"{name}: single-layer batch_first GRU with hidden size in {{8,16,32,64}}")
@@ -105,6 +129,39 @@ def gru_last_hidden(x, gru):
     _check_gru(gru, "gru_last_hidden")
     gi = torch.nn.functional.linear(x, gru.weight_ih_l0, gru.bias_ih_l0)
     return _GRURecurrence.apply(gi, gru.weight_hh_l0, gru.bias_hh_l0)
+
+
+def gru_sequence(x, gru):
+    """Every hidden state (B, L, H) of a single-layer batch_first GRU started from zeros (nn.GRU's `output`): the DIEN
+    paper's interest extractor.  Same kernels as gru_last_hidden; the backward takes a gradient for every h_t."""
+    _check_gru(gru, "gru_sequence")
+    gi = torch.nn.functional.linear(x, gru.weight_ih_l0, gru.bias_ih_l0)
+    return _GRUSequence.apply(gi, gru.weight_hh_l0, gru.bias_hh_l0)
+
+
+class _DIENAux(torch.autograd.Function):
+    """rs_dien_aux_fwd / rs_dien_aux_bwd; the upstream gradient stays on the device."""
+
+    @staticmethod
+    def forward(ctx, h, pos, neg):
+        from . import ops
+        loss, sig = ops.dien_aux_fwd(h, pos, neg)
+        ctx.save_for_backward(h, pos, neg, sig)
+        return loss
+
+    @staticmethod
+    def backward(ctx, g):
+        from . import ops
+        h, pos, neg, sig = ctx.saved_tensors
+        return ops.dien_aux_bwd(h, pos, neg, sig, g.reshape(1))
+
+
+def dien_aux_loss(h, pos, neg):
+    """The DIEN paper's auxiliary loss (eq. 5, inner-product form), the mean over the B (L-1) pairs (b, t < L-1) of
+    softplus(-<h_t, pos_t>) + softplus(<h_t, neg_t>): h (B, L, D) extractor states, pos (B, L-1, D) the embeddings of the
+    next clicked items e_{t+1}, neg (B, L-1, D) those of drawn negatives.  Strided views (slices of one lookup) are read
+    in place.  D in {16, 32, 64}."""
+    return _DIENAux.apply(h, pos, neg)
 
 
 class _AUGRURecurrence(torch.autograd.Function):

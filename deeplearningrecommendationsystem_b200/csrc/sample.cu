@@ -7,6 +7,9 @@
 // (sample index, attempt block, call epoch) -- so every (user, slot) is a pure function of (seed, epoch) regardless of
 // scheduling, and the numpy restatement in oracle/sampling.py reproduces it bit for bit.
 //
+// rs_dien_negatives draws the negatives of DIEN's auxiliary loss on the same stream (an extension: the reference has no
+// auxiliary loss), one slot per (sample, history position), redrawn while equal to the clicked item.
+//
 // rs_assemble_features is data/reader.py:98-101 (`pd.merge` with the user and the item side-feature tables):
 // row b = [user, item, user_feat[user, :], item_feat[item, :]] as fp32, one coalesced pass.
 #include "common.cuh"
@@ -71,6 +74,34 @@ __global__ void sample_negatives_kernel(const int64_t *__restrict__ excl, int64_
   }
 }
 
+// DIEN auxiliary-loss negatives: slot s = b (L-1) + t draws a uniform item for position t+1 of sample b, redrawn while it
+// equals hist[b, t+1].  The epoch is read from device memory, so a graph-replayed step that advances it on the device
+// draws a fresh set on every replay.
+__global__ void dien_negatives_kernel(const int64_t *__restrict__ hist, int64_t B, int L, int64_t num_item, uint32_t seed_lo,
+                                      uint32_t seed_hi, const int64_t *__restrict__ epoch_p, int64_t *__restrict__ neg,
+                                      int32_t *status) {
+  const int64_t per = L - 1, total = B * per;
+  const uint32_t epoch = (uint32_t)*epoch_p;
+  for (int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; s < total; s += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t b = s / per, t = s - b * per;
+    const int64_t pos = clamp_id(hist[b * L + t + 1], num_item, status);
+    int64_t item = -1;
+    for (uint32_t blk = 0; blk < MAX_BLOCKS && item < 0; ++blk) {
+      Philox p = philox4x32_10((uint32_t)s, (uint32_t)(s >> 32), blk, epoch, seed_lo, seed_hi);
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {
+        const int64_t cand = (int64_t)(((uint64_t)p.c[j] * (uint64_t)num_item) >> 32);
+        if (item < 0 && cand != pos) item = cand;
+      }
+    }
+    if (item < 0) {
+      atomicOr(status, 8);
+      item = pos + 1 < num_item ? pos + 1 : 0;
+    }
+    neg[s] = item;
+  }
+}
+
 __global__ void assemble_features_kernel(const int64_t *__restrict__ users, const int64_t *__restrict__ items,
                                          const float *__restrict__ user_feat, int64_t num_user, int FU,
                                          const float *__restrict__ item_feat, int64_t num_item, int FI, int64_t B,
@@ -114,6 +145,23 @@ RS_API int rs_sample_negatives(const int64_t *excluded_keys, int64_t num_exclude
   sample_negatives_kernel<<<(unsigned)(blocks < cap ? blocks : cap), 256, 0, (cudaStream_t)stream>>>(
       excluded_keys, num_excluded, num_user, num_item, num_negatives, (uint32_t)seed, (uint32_t)(seed >> 32), epoch, out_users,
       out_items, status);
+  RS_CHECK_LAUNCH();
+  return 0;
+}
+
+RS_API int rs_dien_negatives(const int64_t *hist, int64_t B, int32_t L, int64_t num_item, uint64_t seed, const int64_t *epoch,
+                             int64_t *neg, int32_t *status, void *stream) {
+  using namespace rs;
+  RS_CHECK_ARG(B >= 0 && L >= 1, RS_E_ARG, "rs_dien_negatives: B=%lld L=%d", (long long)B, L);
+  RS_CHECK_ARG(num_item >= 2 && num_item < (1ll << 32), RS_E_ARG, "rs_dien_negatives: num_item=%lld outside [2, 2^32)",
+               (long long)num_item);
+  const int64_t total = B * (L - 1);
+  if (total == 0) return 0;
+  RS_CHECK_ARG(hist && epoch && neg && status, RS_E_ARG, "rs_dien_negatives: null hist/epoch/neg/status");
+  int64_t blocks = (total + 255) / 256;
+  int64_t cap = (int64_t)num_sms() * 16;
+  dien_negatives_kernel<<<(unsigned)(blocks < cap ? blocks : cap), 256, 0, (cudaStream_t)stream>>>(
+      hist, B, L, num_item, (uint32_t)seed, (uint32_t)(seed >> 32), epoch, neg, status);
   RS_CHECK_LAUNCH();
   return 0;
 }

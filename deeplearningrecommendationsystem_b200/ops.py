@@ -89,6 +89,8 @@ def check_status(device=None):
         if v & 16:
             raise RuntimeError("row exchange: an owner was asked for more rows than its receive capacity "
                                "(raise recv_slack of the DeviceRowExchange); the step's update is incomplete")
+        if v & 8:
+            raise RuntimeError("dien_negatives: a slot found no item distinct from its positive in 65536 attempts")
         raise IndexError("index out of range in embedding lookup")
 
 
@@ -796,6 +798,74 @@ def augru_bwd(w_hh, att, h_all, gates, g_h_all=None, g_h_last=None):
                    "rs_augru_bwd")
     _count()
     return d_gi, d_gh, d_att
+
+
+def _sample_rows(t, name, D):
+    """per-sample stride (elements) of a (B, n, D) float32 CUDA view whose rows are contiguous inside a sample"""
+    _need_cuda(t)
+    if t.dtype != torch.float32 or t.dim() != 3 or t.shape[2] != D or t.stride(2) != 1 or (t.shape[1] > 1 and t.stride(1) != D):
+        raise ValueError(f"{name}: expected a float32 (B, n, {D}) view with contiguous rows, got {t.dtype} {tuple(t.shape)} "
+                         f"strides {t.stride()}")
+    return t.stride(0)
+
+
+def dien_aux_fwd(h, pos, neg):
+    """DIEN auxiliary loss: h (B, L, D) extractor states, pos / neg (B, L-1, D) next-item / negative rows (strided views are
+    read in place) -> loss (0-d, mean over the B (L-1) pairs), sig (B, L-1, 2) = (sigma(x+) - 1, sigma(x-))."""
+    B, L, D = h.shape
+    sh, sp, sn = _sample_rows(h, "dien_aux_fwd h", D), _sample_rows(pos, "dien_aux_fwd pos", D), _sample_rows(neg, "dien_aux_fwd neg", D)
+    if tuple(pos.shape) != (B, L - 1, D) or tuple(neg.shape) != (B, L - 1, D):
+        raise ValueError(f"dien_aux_fwd: pos {tuple(pos.shape)} / neg {tuple(neg.shape)}, expected {(B, L - 1, D)}")
+    sig = torch.empty(B, L - 1, 2, dtype=torch.float32, device=h.device)
+    loss = torch.zeros((), dtype=torch.float32, device=h.device)
+    if B == 0:
+        return loss, sig
+    ws = torch.empty(1024, dtype=torch.float32, device=h.device)
+    with _timed("dien_aux_fwd"):
+        _lib.check(_lib.load().rs_dien_aux_fwd(h.data_ptr(), sh, pos.data_ptr(), sp, neg.data_ptr(), sn, B, L, D, sig.data_ptr(),
+                                               loss.data_ptr(), ws.data_ptr(), _stream()), "rs_dien_aux_fwd")
+    _count(2)
+    return loss, sig
+
+
+def dien_aux_bwd(h, pos, neg, sig, g):
+    """-> dh (B, L, D) (zero at t = L-1), d_pos, d_neg (B, L-1, D) for an upstream gradient g (device scalar tensor)."""
+    B, L, D = h.shape
+    sh, sp, sn = _sample_rows(h, "dien_aux_bwd h", D), _sample_rows(pos, "dien_aux_bwd pos", D), _sample_rows(neg, "dien_aux_bwd neg", D)
+    sig, g = _f32(sig), _f32(g)
+    _need_cuda(sig, g)
+    if g.numel() != 1:
+        raise ValueError("dien_aux_bwd: g must be a scalar")
+    dh = torch.empty(B, L, D, dtype=torch.float32, device=h.device)
+    d_pos = torch.empty(B, L - 1, D, dtype=torch.float32, device=h.device)
+    d_neg = torch.empty_like(d_pos)
+    if B == 0:
+        return dh, d_pos, d_neg
+    with _timed("dien_aux_bwd"):
+        _lib.check(_lib.load().rs_dien_aux_bwd(h.data_ptr(), sh, pos.data_ptr(), sp, neg.data_ptr(), sn, B, L, D, sig.data_ptr(),
+                                               g.data_ptr(), dh.data_ptr(), d_pos.data_ptr(), d_neg.data_ptr(), _stream()),
+                   "rs_dien_aux_bwd")
+    _count()
+    return dh, d_pos, d_neg
+
+
+def dien_negatives(hist, num_items, seed, epoch):
+    """Negatives of the DIEN auxiliary loss: (B, L-1) int64, slot (b, t) uniform over [0, num_items) and != hist[b, t+1]
+    (rs_sample_negatives' Philox stream, counter (b (L-1) + t, attempt block, epoch)).  epoch: int64 device scalar read by
+    the kernel (the caller advances it).  Out-of-range history ids set the status word's bit 0, as a lookup does."""
+    hist = _i64(hist)
+    _need_cuda(hist, epoch)
+    if epoch.dtype != torch.int64 or epoch.numel() != 1:
+        raise ValueError("dien_negatives: epoch must be an int64 device scalar")
+    B, L = hist.shape
+    neg = torch.empty(B, max(L - 1, 0), dtype=torch.int64, device=hist.device)
+    if neg.numel():
+        with _timed("dien_negatives"):
+            _lib.check(_lib.load().rs_dien_negatives(hist.data_ptr(), B, L, int(num_items), seed & (2 ** 64 - 1), epoch.data_ptr(),
+                                                     neg.data_ptr(), status_word(hist.device).data_ptr(), _stream()),
+                       "rs_dien_negatives")
+        _count()
+    return neg
 
 
 def afm_fwd(E, W, b, h, want_attw=True):

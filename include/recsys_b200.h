@@ -426,6 +426,21 @@ int rs_augru_fwd(const float *gi, const float *att, int64_t B, int32_t L, int32_
 int rs_augru_bwd(const float *w_hh, const float *att, const float *h_all, const float *gates, const float *g_h_all,
                  const float *g_h_last, int64_t B, int32_t L, int32_t H, float *d_gi, float *d_gh, float *d_att, void *stream);
 
+/* ---- DIEN auxiliary loss (the DIEN paper's eq. 5, inner-product form; an extension, the reference has none).
+ * h (B, L, D): the interest extractor's states; pos / neg (B, L-1, D): e_{t+1} and the negative e^_{t+1}.  Each operand is
+ * read in place from a strided view: row t of sample b at base + b * stride + t * D floats (base 16-byte aligned, stride a
+ * multiple of 4).  With x+ = <h_t, e_{t+1}>, x- = <h_t, e^_{t+1}> for t = 0..L-2:
+ *   rs_dien_aux_fwd  *loss = 1/(B (L-1)) sum [softplus(-x+) + softplus(x-)]  (0 when L == 1), reduced in a fixed order through
+ *                    ws (>= 1024 floats): bit-reproducible.  sig (B, L-1, 2) = (sigma(x+) - 1, sigma(x-)) per pair.
+ *   rs_dien_aux_bwd  with c = *g / (B (L-1)) (g: device scalar): dh (B, L, D) = c [sig0 e_{t+1} + sig1 e^_{t+1}], zero at
+ *                    t = L-1; d_pos (B, L-1, D) = c sig0 h_t; d_neg (B, L-1, D) = c sig1 h_t.  Outputs contiguous.
+ * D in {16, 32, 64} (RS_E_UNSUPPORTED otherwise).  B == 0 is a no-op. */
+int rs_dien_aux_fwd(const float *h, int64_t h_stride, const float *pos, int64_t pos_stride, const float *neg, int64_t neg_stride,
+                    int64_t B, int32_t L, int32_t D, float *sig, float *loss, float *ws, void *stream);
+int rs_dien_aux_bwd(const float *h, int64_t h_stride, const float *pos, int64_t pos_stride, const float *neg, int64_t neg_stride,
+                    int64_t B, int32_t L, int32_t D, const float *sig, const float *g, float *dh, float *d_pos, float *d_neg,
+                    void *stream);
+
 /* ---- C (M, N) = A^T B for row-major A (K, M), B (K, N): PNN "out" mode's batch-collapsed outer product
  * p = S^T S, S = sum_f e_f (model/pnn.py:69-72), on tcgen05 tensor cores with a 3xTF32 operand split (hi/lo) and fp32
  * accumulation in tensor memory, so the result stays within the path's 1e-5 bar.  M <= 128, N <= 256. */
@@ -487,6 +502,13 @@ int rs_mf_rank(const float *user_rows, const float *item_rows, int64_t num_users
 int rs_sample_negatives(const int64_t *excluded_keys, int64_t num_excluded, int64_t num_user, int64_t num_item,
                         int32_t num_negatives, uint64_t seed, uint32_t epoch, int64_t *out_users, int64_t *out_items,
                         int32_t *status, void *stream);
+/* Negatives of the DIEN auxiliary loss, same stream: slot s = b (L-1) + t of neg (B, L-1) is drawn with counter
+ * (s lo, s hi, attempt block, (uint32) *epoch), redrawn while it equals hist[b, t+1] (hist (B, L) contiguous; an
+ * out-of-range id is clamped and sets status bit 0).  epoch: DEVICE int64 scalar, read by the kernel, so a captured step
+ * that advances it on the device draws fresh negatives on every replay.  num_item >= 2.  status |= 8 if a slot found no
+ * item in 65536 attempts (it then takes hist + 1 mod num_item). */
+int rs_dien_negatives(const int64_t *hist, int64_t B, int32_t L, int64_t num_item, uint64_t seed, const int64_t *epoch,
+                      int64_t *neg, int32_t *status, void *stream);
 
 /* ---- feature-matrix assembly (data/reader.py:98-101, the two pd.merge calls): out (B, 2 + user_width + item_width)
  * fp32 rows [user, item, user_feat[user, :], item_feat[item, :]].  status |= 1 on an out-of-range id. */
