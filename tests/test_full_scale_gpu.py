@@ -37,8 +37,11 @@ def sparse_sgd_reference(kind, rows, inv, y, lr, bias=None, dim=None, chunk=4096
     rows (U, W): the distinct table rows the batch looks up, as they were before the step.  inv (B, F): index into
     `rows` of lookup (b, i).  y: B labels.  bias: the scalar bias before the step (FM / FFM), None for MF (no bias).
     dim: D of the FFM row (F slots of D floats).  Logits follow oracle.nfield.fm_logit / ffm_logit and oracle.ml100k.mf.
-    Returns a dict: pred (B,), loss, rows (U, W) after the step, grad (U, W) = summed gradient, absg (U, W) = summed
-    |gradient terms| of each element, bias after the step (None for MF).  Stock torch ops only; runs where `rows` is.
+    Returns a dict: pred (B,), loss, rows (U, W) after the step, grad (U, W) = summed gradient, absg (U, W) = the L1 mass
+    the element's fp32 gradient is formed from: the sum over its terms of |d loss / d logit| times the L1 mass of the
+    Jacobian element (FM: sum_f e_f - e_i is formed from an fp32 sum over the fields that can cancel, so its mass is
+    sum_f |e_f|, not its value; FFM and MF: a single table value), bias after the step (None for MF).  Stock torch ops
+    only; runs where `rows` is.
     """
     nb, F = inv.shape
     U, W = rows.shape
@@ -56,10 +59,12 @@ def sparse_sgd_reference(kind, rows, inv, y, lr, bias=None, dim=None, chunk=4096
         idx = inv[s:s + chunk]
         c = idx.shape[0]
         E = rows[idx].double()                                     # (c, F, W)
+        mass = None
         if kind == "fm":
             tot = E.sum(1)
             logit = 0.5 * (tot * tot - (E * E).sum(1)).sum(1)
             jac = tot.unsqueeze(1) - E                             # d logit / d e_i = sum_f e_f - e_i
+            mass = E.abs().sum(1, keepdim=True).expand_as(E)      # the fp32 sum of the F rows can cancel
         elif kind == "mf":
             logit = (E[:, 0] * E[:, 1]).sum(1)
             jac = E.flip(1)                                        # d <u, v> / du = v, d / dv = u
@@ -77,10 +82,10 @@ def sparse_sgd_reference(kind, rows, inv, y, lr, bias=None, dim=None, chunk=4096
         terms = (g[:, None, None] * jac).reshape(-1, W)
         flat = idx.reshape(-1)
         grad.index_add_(0, flat, terms)
-        absg.index_add_(0, flat, terms.abs())
+        absg.index_add_(0, flat, terms.abs() if kind != "fm" else (g.abs()[:, None, None] * mass).reshape(-1, W))
         gsum += g.sum()
         pred[s:s + c] = p
-        del E, jac, terms
+        del E, jac, terms, mass
     return {"pred": pred, "loss": loss / nb, "rows": rows.double() - lr * grad, "grad": grad, "absg": absg,
             "bias": None if bias is None else b0 - lr * float(gsum)}
 
@@ -156,30 +161,39 @@ def make_batch(cards, dist, seed, nb=B):
     return ids, y
 
 
+def guard_sample(cards, seed, device):
+    """sorted distinct rows of the concatenated table: a seeded sample of about 1.1 GUARD_SAMPLE rows spread over every
+    field in proportion to its size, at least 1000 (or all) rows of each"""
+    total = sum(cards)
+    g = torch.Generator(device=device).manual_seed(seed)
+    want = int(GUARD_SAMPLE * 1.1)
+    parts, o = [], 0
+    for c in cards:
+        k = max(1000, want * c // total)
+        parts.append(o + (torch.arange(c, device=device) if k >= c else torch.randint(0, c, (k,), generator=g, device=device)))
+        o += c
+    return torch.unique(torch.cat(parts))
+
+
+def wrap_images(rows, base, width):
+    """the rows that hold float offset (o mod 2^32) and (o mod 2^31) and byte offset (4 o mod 2^32) from `base`, where
+    o = (rows - base) * width is the float offset of each row from that base: where a 32-bit offset would land"""
+    o = (rows - base) * width
+    return torch.cat([base + wrapped // width for wrapped in (o % (1 << 32), o % (1 << 31), (4 * o) % (1 << 32) // 4)])
+
+
 def guard_rows(cards, width, uniq, seed):
     """Sorted distinct global rows the step must leave bit-identical: a seeded sample of >= GUARD_SAMPLE rows spread over
-    every field, plus the wrap images of every touched row -- the rows that hold float offset (r W mod 2^32) and
-    (r W mod 2^31) and byte offset (4 r W mod 2^32), relative to the concatenated table and to the row's own field --
-    minus the touched rows themselves."""
+    every field, plus the wrap images of every touched row relative to the concatenated table and to the row's own
+    field, minus the touched rows themselves."""
     dev = uniq.device
     total = sum(cards)
     offs = torch.tensor([sum(cards[:k]) for k in range(len(cards))], device=dev)
-    g = torch.Generator(device=dev).manual_seed(seed)
-    want = int(GUARD_SAMPLE * 1.1)
-    parts = []
-    for o, c in zip(offs.tolist(), cards):
-        k = max(1000, want * c // total)
-        parts.append(o + (torch.arange(c, device=dev) if k >= c else torch.randint(0, c, (k,), generator=g, device=dev)))
-    sample = torch.unique(torch.cat(parts))
+    sample = guard_sample(cards, seed, dev)
     sample = sample[~torch.isin(sample, uniq)]
     assert sample.numel() >= GUARD_SAMPLE, sample.numel()
     base = offs[torch.searchsorted(offs, uniq, right=True) - 1]
-    images = []
-    for b0 in (torch.zeros_like(uniq), base):
-        o = (uniq - b0) * width                                   # float offset of the row from that base
-        for wrapped in (o % (1 << 32), o % (1 << 31), (4 * o) % (1 << 32) // 4):
-            images.append(b0 + wrapped // width)
-    images = torch.unique(torch.cat(images))
+    images = torch.unique(torch.cat([wrap_images(uniq, b0, width) for b0 in (torch.zeros_like(uniq), base)]))
     images = images[~torch.isin(images, uniq)]
     assert images.numel() == 0 or int(images.max()) < total
     return torch.unique(torch.cat([sample, images])), int(images.numel())
@@ -187,8 +201,9 @@ def guard_rows(cards, width, uniq, seed):
 
 # ---------------------------------------------------------------------------------------------- per-step checks
 def assert_rows_match(got, ref, lr, what, chunk=1 << 17):
-    """|w_gpu - w64| <= 1e-6 |w64| + lr (1e-5 |g64| + 4 eps32 S) for every element (S = sum of |gradient terms|): the
-    scaled floor of test_segment_grad_and_sgd -- a fp32 sum of n terms carries a few ulp of their L1 mass."""
+    """|w_gpu - w64| <= 1e-6 |w64| + lr (1e-5 |g64| + 4 eps32 S) for every element (S = ref["absg"], the L1 mass the
+    gradient is formed from): the scaled floor of test_segment_grad_and_sgd -- a fp32 sum of n terms carries a few ulp of
+    their L1 mass."""
     worst = 0.0
     for s in range(0, got.shape[0], chunk):
         w64, g64, S = ref["rows"][s:s + chunk], ref["grad"][s:s + chunk], ref["absg"][s:s + chunk]
@@ -266,12 +281,12 @@ def need_free(gb):
     return f"{free / 1e9:.1f} GB free ({torch.cuda.memory_allocated() / 1e9:.1f} GB held by this process)"
 
 
-def _field_trainer(model):
-    """Trainer + FusedRowOptimizer(kind="sgd") as bench.py builds them"""
+def _field_trainer(model, kind="sgd", weight_decay=0.0):
+    """Trainer + FusedRowOptimizer (lr LR; SGD on the bias) as bench.py builds them"""
     from deeplearningrecommendationsystem_b200.optim import FusedRowOptimizer
     from deeplearningrecommendationsystem_b200.trainer import Trainer
     dense = torch.optim.SGD([model.bias], lr=LR) if model.bias.requires_grad else None
-    return Trainer(model, torch.nn.BCELoss(), FusedRowOptimizer(model, dense, lr=LR, kind="sgd"))
+    return Trainer(model, torch.nn.BCELoss(), FusedRowOptimizer(model, dense, lr=LR, kind=kind, weight_decay=weight_decay))
 
 
 # Device memory each case needs: the table, the step's own buffers (FFM: 2.8 GB Jacobian stash), the sparse reference
