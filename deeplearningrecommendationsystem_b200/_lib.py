@@ -146,6 +146,9 @@ SIGNATURES = {
     "rs_gemm_tn_ws_bytes": [_L, _I, _I, _PP(_Z)],
     "rs_gemm_tn_3xtf32": [_P, _P, _L, _I, _I, _P, _P, _Z, _P],
     "rs_gemm_nt_3xtf32": [_PP(rs_gemm_nt), _P],
+    "rs_pnn_outer_ws_bytes": [_L, _I, _I, _PP(_Z), _PP(_Z)],
+    "rs_pnn_outer_fwd": [_P, _L, _I, _I, _I, _P, _P, _P, _P, _P, _Z, _P],
+    "rs_pnn_outer_bwd": [_P, _P, _L, _I, _I, _P, _P, _P, _P, _P, _Z, _P],
     "rs_gru_fwd": [_P, _L, _I, _I, _P, _P, _P, _P, _P],
     "rs_gru_bwd": [_P, _P, _P, _P, _P, _L, _I, _I, _P, _P, _P],
     "rs_augru_fwd": [_P, _P, _L, _I, _I, _P, _P, _P, _P, _P],

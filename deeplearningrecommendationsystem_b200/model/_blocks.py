@@ -326,6 +326,25 @@ class OuterPooled(torch.autograd.Function):
         return S @ (G + G.t())
 
 
+class OuterProduct(torch.autograd.Function):
+    """lp = W vec(s s^T) + b per sample, s = sum_f E[:, f] -- the PNN paper's outer-product layer with sum pooling (an
+    extension: the reference's "out" mode is the batch-collapsed OuterPooled).  Forward and backward are one C-ABI call
+    each (rs_pnn_outer_fwd / _bwd on tcgen05); every field row of a sample receives the same gradient dS."""
+
+    @staticmethod
+    def forward(ctx, E, W, b):
+        lp, S = ops.pnn_outer_fwd(E, W, b)
+        ctx.save_for_backward(S, W)
+        ctx.F = E.shape[1]
+        return lp
+
+    @staticmethod
+    def backward(ctx, g):
+        S, W = ctx.saved_tensors
+        dS, dW, db = ops.pnn_outer_bwd(S, g.contiguous(), W)
+        return dS.unsqueeze(1).expand(-1, ctx.F, -1), dW, db
+
+
 class FFMDense(torch.autograd.Function):
     """sum_{i<j} <T[i, field(j)], T[j, field(i)]> over dense T (B, F, NF, D)     model/ffm.py:61-82"""
 

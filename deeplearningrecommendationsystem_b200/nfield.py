@@ -623,22 +623,37 @@ class _EmbedModel(_FieldModel):
 
 class FieldPNN(_EmbedModel):
     """Inner-product PNN over F id-fields (reference model/pnn.py:55-77,111-131 generalised from six features):
-    lz = Linear(F*D, H0)(concat), lp = Linear(F(F-1)/2, H0)(inner products), ReLU tower, Linear(H[-1], 1), sigmoid."""
+    lz = Linear(F*D, H0)(concat), lp = Linear(F(F-1)/2, H0)(inner products), ReLU tower, Linear(H[-1], 1), sigmoid.
+
+    product="outer": the PNN paper's outer-product layer with sum pooling instead (an extension; the reference's "out"
+    mode collapses the batch, see model.PNN): lp = Linear(D*D, H0)(vec(s s^T)) per sample with s = sum_f e_f, on the
+    tensor cores (rs_pnn_outer_fwd / _bwd).  linear2.weight is then (H0, D*D); D in {16, 32, 64}, H0 a multiple of 16
+    up to 512."""
 
     use_bias = False
 
-    def __init__(self, cardinalities, embed_dim, hidden_units, fused=True, seed=None, device=None, sharded=False, group=None, **kw):
+    def __init__(self, cardinalities, embed_dim, hidden_units, fused=True, seed=None, device=None, sharded=False, group=None,
+                 product="inner", **kw):
+        if product not in ("inner", "outer"):
+            raise ValueError(f'product must be "inner" or "outer", got {product!r}')
         super().__init__(cardinalities, embed_dim, embed_dim, fused, seed, device, sharded, group, **kw)
         F = self.F
+        self.product = product
         self.bias.requires_grad_(False)
         self.linear1 = nn.Linear(F * embed_dim, hidden_units[0], device=device)
-        self.linear2 = nn.Linear(F * (F - 1) // 2, hidden_units[0], device=device)
+        self.linear2 = nn.Linear(F * (F - 1) // 2 if product == "inner" else embed_dim * embed_dim, hidden_units[0], device=device)
         self.dnn_network = nn.ModuleList([nn.Linear(a, b, device=device) for a, b in zip(hidden_units[:-1], hidden_units[1:])])
         self.output = nn.Linear(hidden_units[-1], 1, device=device)
 
     def forward(self, ids):
-        concat, pairs = self.embed(ids, want_pairs=True)
-        h = self.linear1(concat) + self.linear2(pairs)
+        if self.product == "outer":
+            from .model._blocks import OuterProduct
+            concat, _ = self.embed(ids)
+            lp = OuterProduct.apply(concat.view(ids.shape[0], self.F, self.width), self.linear2.weight, self.linear2.bias)
+            h = self.linear1(concat) + lp
+        else:
+            concat, pairs = self.embed(ids, want_pairs=True)
+            h = self.linear1(concat) + self.linear2(pairs)
         for layer in self.dnn_network:
             h = torch.relu(layer(h))
         return torch.sigmoid(self.output(h)).view(-1, 1)

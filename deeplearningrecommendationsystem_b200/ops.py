@@ -1089,6 +1089,56 @@ def gemm_tn(A, B):
     return out
 
 
+def _pnn_outer_ws(B, D, H0, device, which):
+    """the workspace of rs_pnn_outer_fwd (which=0) / _bwd (which=1), allocated per call through torch: a captured step
+    keeps its own block from the graph's pool instead of a cache that a later eager call could replace"""
+    fwd, bwd = C.c_size_t(0), C.c_size_t(0)
+    _lib.check(_lib.load().rs_pnn_outer_ws_bytes(B, D, H0, C.byref(fwd), C.byref(bwd)), "rs_pnn_outer_ws_bytes")
+    n = (fwd, bwd)[which].value
+    return torch.empty(max(n, 16), dtype=torch.uint8, device=device), n
+
+
+def pnn_outer_fwd(E, W, b):
+    """The PNN paper's outer-product layer: E (B, F, D), W (H0, D*D), b (H0) -> lp (B, H0), S (B, D) with s = sum_f E[:, f],
+    lp = Linear(D*D, H0)(vec(s s^T)) per sample (tcgen05, 3xTF32).  D in {16, 32, 64}, H0 a multiple of 16 up to 512."""
+    E, W, b = _f32(E), _f32(W), _f32(b)
+    _need_cuda(E, W, b)
+    B, F, D = E.shape
+    H0 = W.shape[0]
+    if tuple(W.shape) != (H0, D * D) or tuple(b.shape) != (H0,):
+        raise ValueError(f"pnn_outer_fwd: W must be ({H0}, {D * D}) and b ({H0},), got {tuple(W.shape)} and {tuple(b.shape)}")
+    ws, n = _pnn_outer_ws(B, D, H0, E.device, 0)
+    lp = torch.empty(B, H0, dtype=torch.float32, device=E.device)
+    S = torch.empty(B, D, dtype=torch.float32, device=E.device)
+    if B == 0:
+        return lp, S
+    with _timed("pnn_outer_fwd"):
+        _lib.check(_lib.load().rs_pnn_outer_fwd(E.data_ptr(), B, F, D, H0, W.data_ptr(), b.data_ptr(), lp.data_ptr(), S.data_ptr(),
+                                                ws.data_ptr(), n, _stream()), "rs_pnn_outer_fwd")
+    _count()
+    return lp, S
+
+
+def pnn_outer_bwd(S, g, W):
+    """S (B, D) from pnn_outer_fwd, g = d loss / d lp (B, H0), W (H0, D*D) -> dS (B, D) (the gradient of every field row),
+    dW (H0, D*D), db (H0); dW and db are slab partials added in slab order (bit-reproducible)."""
+    S, g, W = _f32(S), _f32(g), _f32(W)
+    _need_cuda(S, g, W)
+    B, D = S.shape
+    H0 = W.shape[0]
+    ws, n = _pnn_outer_ws(B, D, H0, S.device, 1)
+    dS = torch.empty(B, D, dtype=torch.float32, device=S.device)
+    if B == 0:
+        return dS, torch.zeros(H0, D * D, dtype=torch.float32, device=S.device), torch.zeros(H0, dtype=torch.float32, device=S.device)
+    dW = torch.empty(H0, D * D, dtype=torch.float32, device=S.device)
+    db = torch.empty(H0, dtype=torch.float32, device=S.device)
+    with _timed("pnn_outer_bwd"):
+        _lib.check(_lib.load().rs_pnn_outer_bwd(S.data_ptr(), g.data_ptr(), B, D, H0, W.data_ptr(), dS.data_ptr(), dW.data_ptr(),
+                                                db.data_ptr(), ws.data_ptr(), n, _stream()), "rs_pnn_outer_bwd")
+    _count()
+    return dS, dW, db
+
+
 def gemm_nt(A, W, bias=None, rowbias=None, rb_group=1, relu=False, mask=None, M=None, a_rows=None):
     """epilogue(A W^T) on tcgen05 (3xTF32).  A (M, K) contiguous, or -- with a_rows=(group, group_stride, lda) -- a
     strided view whose row r lives at A.data_ptr + (r // group)*group_stride + (r % group)*lda floats.

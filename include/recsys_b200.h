@@ -448,6 +448,23 @@ int rs_gemm_tn_ws_bytes(int64_t K, int32_t M, int32_t N, size_t *bytes);
 int rs_gemm_tn_3xtf32(const float *A, const float *B, int64_t K, int32_t M, int32_t N, float *C, float *ws,
                       size_t ws_bytes, void *stream);
 
+/* ---- Per-sample outer-product layer of the PNN paper (OPNN with sum pooling; an extension: the reference's "out" mode
+ * is the batch-collapsed S^T S above).  E (B, F, D) field rows, W (H0, D*D) and bias (H0) in torch Linear layout:
+ *   s_b = sum_f E[b, f, :]  (D),   lp[b, h] = sum_{i,j} W[h, i D + j] s_b[i] s_b[j] + bias[h]     i.e. Linear(D*D, H0)(vec(s s^T)).
+ * rs_pnn_outer_fwd writes lp (B, H0) and S (B, D), the s_b the backward takes.  With g = d loss / d lp (B, H0),
+ * rs_pnn_outer_bwd writes
+ *   dS[b, i] = sum_h g[b, h] sum_j (W[h, i D + j] + W[h, j D + i]) s_b[j]   (= d loss / d E[b, f, :] for every f),
+ *   dW[h, i D + j] = sum_b g[b, h] s_b[i] s_b[j],   db[h] = sum_b g[b, h].
+ * tcgen05 tensor cores with a 3xTF32 split and fp32 accumulation in tensor memory; p = s s^T never reaches global memory.
+ * No atomics: results are bit-identical from run to run.  Workspace: rs_pnn_outer_ws_bytes (fwd_bytes: the repacked
+ * weight; bwd_bytes: that plus the per-slab partials of dW, db).  E, S, dS and ws 16-byte aligned, all contiguous.
+ * D in {16, 32, 64} and H0 a multiple of 16 in [16, 512] (RS_E_UNSUPPORTED otherwise); any B >= 0 and F >= 1. */
+int rs_pnn_outer_ws_bytes(int64_t B, int32_t D, int32_t H0, size_t *fwd_bytes, size_t *bwd_bytes);
+int rs_pnn_outer_fwd(const float *E, int64_t B, int32_t F, int32_t D, int32_t H0, const float *W, const float *bias, float *lp,
+                     float *S, void *ws, size_t ws_bytes, void *stream);
+int rs_pnn_outer_bwd(const float *S, const float *g, int64_t B, int32_t D, int32_t H0, const float *W, float *dS, float *dW,
+                     float *db, void *ws, size_t ws_bytes, void *stream);
+
 /* C (M, N) = epilogue(A B^T) on tcgen05 (3xTF32): the DIN / DIEN attention-unit layers over all B*L rows
  * (model/din.py:14-20,43).  A (M, K): row r at A + (r / a_group)*a_group_stride + (r % a_group)*lda when a_group > 0
  * (rows of a (B, L+1, D) gather viewed as B*L history rows), else A + r*lda.  B (N, K) in torch Linear layout, kept
